@@ -2,7 +2,7 @@
 """Benchmark of the variational-layer hot path (BASELINE.json metric: train samples/s & MC-predictive samples/s at
 1/2/4/8 B200; % TC peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Default (`--workload headline`): the configuration the metric's "% TC peak" is quoted on -- BASELINE.json configs[4], the
 widened LRT stack 4096-4096-4096-10 in bf16 at batch 8192 per GPU (tcgen05 / TMEM / TMA kernels; data-parallel over the N
@@ -13,6 +13,9 @@ One step = forward + loss + backward + Adam on one synthetic minibatch (LBBNN-GP
 `--workload NAME` runs one workload alone.  `--impl reference` times the REFERENCE's own classes and `train` function
 (oracle/_ref, built by oracle/make_ref.py from /root/reference) on the host cores.
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for how every field is obtained.
+`--dump-outputs DIR` (LRT training workloads): after the timed steps, rank 0 writes what the last of them left to the
+caller -- the step statistics and the updated parameters -- as DIR/<name>.npy, so that two builds can be compared output
+for output on identical inputs (same arguments, same seeds).
 """
 import argparse
 import json
@@ -26,6 +29,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (os.path.join(ROOT, "bayesian-neural-nets_b200"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np
 import torch
@@ -126,6 +130,36 @@ def make_pool(pool, batch, in_features, classes, seed):
     x = torch.from_numpy(rng.random((pool, batch, in_features), dtype=np.float32))
     y = torch.from_numpy(rng.integers(0, classes, size=(pool, batch))).long()
     return x, y
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed, for output-for-output comparison of two builds
+# ------------------------------------------------------------------------------------------------
+DUMP_LIMIT = 64 << 20       # bytes written in all
+DUMP_SAMPLE = 1 << 20       # entries kept of a larger parameter (the wide stack's 4096 x 4096 weights)
+
+
+def training_outputs(tr, net):
+    """The step statistics [nll, kl_1 .. kl_L] (`stats`) and every updated parameter of the network (`l1.weight_mu`, ...).
+    A parameter of more than DUMP_SAMPLE entries is saved as `<name>.sample`: its flattened entries at DUMP_SAMPLE
+    positions drawn with a fixed seed, the same positions in every run."""
+    out = {"stats": tr.stats.cpu().numpy()}
+    for name, p in net.named_parameters():
+        flat = p.detach().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+            flat, name = flat[torch.from_numpy(pos).to(flat.device)], name + ".sample"
+        out[name] = flat.float().cpu().numpy()
+    return out
+
+
+def dump_outputs(directory, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -472,8 +506,9 @@ class Ctx:
         t.cancel()
 
 
-def bench_lrt(ctx, workload, steps, warmup, unfused=False, cpu_budget_s=15.0):
-    """One LRT training workload (lrt_mnist / lrt_wide) on this run's GPUs; returns the record on rank 0, None elsewhere."""
+def bench_lrt(ctx, workload, steps, warmup, unfused=False, cpu_budget_s=15.0, dump_dir=None):
+    """One LRT training workload (lrt_mnist / lrt_wide) on this run's GPUs; returns the record on rank 0, None elsewhere.
+    dump_dir: rank 0 writes training_outputs() of the last timed step there."""
     import lbbnn
     if os.environ.get("LBBNN_HANG_DUMP"):
         import faulthandler
@@ -525,6 +560,8 @@ def bench_lrt(ctx, workload, steps, warmup, unfused=False, cpu_budget_s=15.0):
     t1 = time.perf_counter()
     ms = e0.elapsed_time(e1)
     _mark(f"timed region done: {ms / args.steps * 1e3:.1f} us/step")
+    if dump_dir and rank == 0:      # now: the end-to-end steps below go on training the same network
+        dump_outputs(dump_dir, training_outputs(tr, net))
 
     # ---- end to end through the public API with host buffers ("e2e") ----------------------------------
     # trainer.step_async(x_host, y_host): every step uploads its batch from pinned host memory (H2D) and its
@@ -1164,7 +1201,7 @@ def bench_module(kind, steps, warmup, eager=False, cpu_budget_s=15.0):
 def run_headline(args):
     """lrt_wide for exactly --steps steps, plus bounded runs of lrt_mnist and mf_mc_predict on the same GPUs (`also`)."""
     ctx = Ctx(args)
-    line = bench_lrt(ctx, "lrt_wide", args.steps, args.warmup, unfused=args.unfused)
+    line = bench_lrt(ctx, "lrt_wide", args.steps, args.warmup, unfused=args.unfused, dump_dir=args.dump_outputs)
     small = bench_lrt(ctx, "lrt_mnist", 2000, 50)
     mc = bench_mc(ctx, args, 8, 3)
     also = {"lrt_mnist": small, "mf_mc_predict": mc}
@@ -1179,7 +1216,7 @@ def run_headline(args):
 
 def run_ours(args):
     ctx = Ctx(args)
-    line = bench_lrt(ctx, args.workload, args.steps, args.warmup, unfused=args.unfused)
+    line = bench_lrt(ctx, args.workload, args.steps, args.warmup, unfused=args.unfused, dump_dir=args.dump_outputs)
     if ctx.rank == 0:
         print(json.dumps(line), flush=True)
     ctx.shutdown()
@@ -1199,7 +1236,11 @@ def main():
     ap.add_argument("--unfused", action="store_true", help="lrt_*: per-layer launch sequence / separate update passes")
     ap.add_argument("--workload", default="headline",
                     choices=["headline"] + sorted(SIZES) + ["mf_mc_predict", "mnf_mnist", "mf_mnist", "vd_mnist"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="headline / lrt_*: write the statistics and updated parameters of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ["headline"] + sorted(SIZES)):
+        ap.error("--dump-outputs covers the LRT training workloads (headline, lrt_mnist, lrt_wide) of --impl ours")
     big = args.workload in ("headline", "lrt_wide")
     if args.steps is None:
         args.steps = 100 if big else (20 if args.workload == "mf_mc_predict" else 2000)

@@ -173,4 +173,25 @@ __host__ __device__ __forceinline__ int64_t ceil_div(int64_t a, int64_t b) { ret
 
 __device__ __forceinline__ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// NVSwitch multicast (NVLS) access through a multicast address: ld_reduce returns the sum over every rank's copy (the
+// reduction happens in the switch), st writes the value to every rank's copy.
+__device__ __forceinline__ float4 mc_ld_reduce4(const float* p) {
+  float4 r;
+  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.v4.f32 {%0, %1, %2, %3}, [%4];"
+               : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p) : "memory");
+  return r;
+}
+__device__ __forceinline__ void mc_st4(float* p, const float v[4]) {
+  asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3])
+               : "memory");
+}
+__device__ __forceinline__ float mc_ld_reduce1(const float* p) {
+  float r;
+  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.f32 %0, [%1];" : "=f"(r) : "l"(p) : "memory");
+  return r;
+}
+__device__ __forceinline__ void mc_st1(float* p, float v) {
+  asm volatile("multimem.st.relaxed.sys.global.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
+}
+
 }  // namespace lbbnn

@@ -766,24 +766,6 @@ __global__ void __launch_bounds__(kThreads) lrt_f32_finalize(const FinalizeArgs 
 // Per rank that is 1/world of the optimiser traffic of the replicated update and (8 + 12) B / weight over NVLink instead of
 // the 2 x 8 B of an all-reduce of (dM, dV) followed by a full update on every rank.  The caller brackets the launch with
 // cross-rank barriers (all ranks' dW GEMMs done before; all stores landed before the parameters are read again).
-__device__ __forceinline__ float4 mc_ld_reduce4(const float* p) {
-  float4 r;
-  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.v4.f32 {%0, %1, %2, %3}, [%4];"
-               : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p) : "memory");
-  return r;
-}
-__device__ __forceinline__ void mc_st4(float* p, const float v[4]) {
-  asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3])
-               : "memory");
-}
-__device__ __forceinline__ float mc_ld_reduce1(const float* p) {
-  float r;
-  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.f32 %0, [%1];" : "=f"(r) : "l"(p) : "memory");
-  return r;
-}
-__device__ __forceinline__ void mc_st1(float* p, float v) {
-  asm volatile("multimem.st.relaxed.sys.global.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
-}
 
 struct DpUpdateArgs {
   const float *mu, *rho, *lam, *bias_mu, *bias_rho;     // this rank's copies (read)

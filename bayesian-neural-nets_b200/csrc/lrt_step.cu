@@ -130,24 +130,6 @@ __device__ __forceinline__ void dp_flag_exchange(const DevStep& a, unsigned epoc
   for (int q = 0; q < a.dp_world; ++q)
     while ((int)(ld_acquire_sys(a.dp_signal[a.dp_rank] + q) - epoch) < 0) {}
 }
-__device__ __forceinline__ float4 mc_ld_reduce4(const float* p) {
-  float4 r;
-  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.v4.f32 {%0, %1, %2, %3}, [%4];"
-               : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p) : "memory");
-  return r;
-}
-__device__ __forceinline__ void mc_st4(float* p, const float v[4]) {
-  asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3])
-               : "memory");
-}
-__device__ __forceinline__ float mc_ld_reduce1(const float* p) {
-  float r;
-  asm volatile("multimem.ld_reduce.relaxed.sys.global.add.f32 %0, [%1];" : "=f"(r) : "l"(p) : "memory");
-  return r;
-}
-__device__ __forceinline__ void mc_st1(float* p, float v) {
-  asm volatile("multimem.st.relaxed.sys.global.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
-}
 
 __device__ __forceinline__ void stamp(const DevStep& a, int& slot) {
   if (a.prof && (int)blockIdx.x == a.prof_cta && threadIdx.x == 0) a.prof[slot] = clock64();

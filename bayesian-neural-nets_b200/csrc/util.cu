@@ -251,6 +251,24 @@ __global__ void adam_prepare_inc(int64_t* __restrict__ step_dev, float lr, float
   coef[1] = (float)sqrt(1.0 - pow((double)b2, t));
 }
 
+// adam_multi_kernel's table search for the data-parallel kernels below: the entry whose [first_block, next first_block) range
+// holds block blk = block_lo + blockIdx.x.  Every thread of the block must call it (it synchronises the block).
+// adam_multi_kernel keeps its own inline copy: through this function its SASS comes out different (same registers).
+__device__ __forceinline__ int adam_table_find(const lbbnn_adam_entry* __restrict__ table, int n_entries, int64_t block_lo,
+                                               int64_t* s_first, int64_t& blk) {
+  const int ns = n_entries < kAdamSmemEntries ? n_entries : kAdamSmemEntries;
+  for (int i = threadIdx.x; i < ns; i += blockDim.x) s_first[i] = table[i].first_block;
+  __syncthreads();
+  int lo = 0, hi = n_entries - 1;
+  blk = block_lo + blockIdx.x;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    const int64_t fb = mid < ns ? s_first[mid] : table[mid].first_block;
+    if (fb <= blk) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
 // The same update over a TABLE of tensors in one launch: block b works on 1024 consecutive elements of the tensor whose
 // [first_block, next first_block) range holds b (binary search over the table, read through L2 by every block).
 __global__ void __launch_bounds__(256) adam_multi_kernel(const lbbnn_adam_entry* __restrict__ table, int n_entries, float b1,
@@ -307,6 +325,59 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const lbbnn_adam_entry*
     for (int j = 0; j < 4; ++j)
       if (e0 + j < e.n) { p[e0 + j] = pv[j]; m[e0 + j] = mv[j]; v[e0 + j] = vv[j]; }
   }
+}
+
+// Data parallel: every entry's parameter lives in one symmetric-memory arena [parameters | packed gradients], its packed
+// gradient grad_offset floats after it.  The pack copies autograd's gradient (entry.grad) of this rank's rows there.
+__global__ void __launch_bounds__(256) adam_pack_kernel(const lbbnn_adam_entry* __restrict__ table, int n_entries,
+                                                        int64_t grad_offset) {
+  __shared__ int64_t s_first[kAdamSmemEntries];
+  int64_t blk;
+  const lbbnn_adam_entry e = table[adam_table_find(table, n_entries, 0, s_first, blk)];
+  const int64_t e0 = (blk - e.first_block) * 1024 + (int64_t)threadIdx.x * 4;
+  if (e0 >= e.n) return;
+  const float* g = e.grad;
+  float* d = e.param + grad_offset;
+  if (e0 + 3 < e.n && aligned16(g) && aligned16(d)) {
+    *reinterpret_cast<float4*>(d + e0) = *reinterpret_cast<const float4*>(g + e0);
+  } else {
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (e0 + j < e.n) d[e0 + j] = g[e0 + j];
+  }
+}
+
+// The sharded update: this rank runs table blocks [block_lo, block_lo + gridDim.x) only.  Per quad: the in-switch sum of the
+// packed gradient over all ranks (multimem.ld_reduce: the reduce-scatter), the Adam step of adam_multi_kernel on this rank's
+// moments, and the new parameter stored to every rank's copy (multimem.st: the all-gather).  Whole quads: the arena pads each
+// tensor to 4 floats with zeros, a zero gradient keeps a zero moment and a zero parameter, so the pads stay zero.
+__global__ void __launch_bounds__(256) adam_multi_dp_kernel(const lbbnn_adam_entry* __restrict__ table, int n_entries,
+                                                            int64_t block_lo, const float* __restrict__ arena, float* arena_mc,
+                                                            int64_t grad_offset, float b1, float b2, float eps,
+                                                            const float* __restrict__ coef) {
+  __shared__ int64_t s_first[kAdamSmemEntries];
+  int64_t blk;
+  const lbbnn_adam_entry e = table[adam_table_find(table, n_entries, block_lo, s_first, blk)];
+  const float step_size = __ldg(coef) * e.lr_scale, bc2_sqrt = __ldg(coef + 1);
+  const int64_t e0 = (blk - e.first_block) * 1024 + (int64_t)threadIdx.x * 4;
+  if (e0 >= e.n) return;
+  const int64_t off = (e.param - arena) + e0;              // float offset of this quad in the arena (a multiple of 4)
+  const float4 gq = mc_ld_reduce4(arena_mc + off + grad_offset);
+  const float4 a = *reinterpret_cast<const float4*>(e.param + e0);
+  const float4 c = *reinterpret_cast<const float4*>(e.exp_avg + e0), d = *reinterpret_cast<const float4*>(e.exp_avg_sq + e0);
+  float pv[4] = {a.x, a.y, a.z, a.w}, gv[4] = {gq.x, gq.y, gq.z, gq.w};
+  float mv[4] = {c.x, c.y, c.z, c.w}, vv[4] = {d.x, d.y, d.z, d.w};
+  const float inv_bc2 = 1.0f / bc2_sqrt;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    mv[j] = mv[j] + (gv[j] - mv[j]) * (1.0f - b1);
+    vv[j] = b2 * vv[j] + (1.0f - b2) * gv[j] * gv[j];
+    const float denom = fmaf(sqrtf(vv[j]), inv_bc2, eps);
+    pv[j] -= step_size * __fdividef(mv[j], denom);
+  }
+  *reinterpret_cast<float4*>(e.exp_avg + e0) = make_float4(mv[0], mv[1], mv[2], mv[3]);
+  *reinterpret_cast<float4*>(e.exp_avg_sq + e0) = make_float4(vv[0], vv[1], vv[2], vv[3]);
+  mc_st4(arena_mc + off, pv);
 }
 
 __global__ void counter_inc_kernel(int64_t* c) { *c += 1; }
@@ -452,4 +523,28 @@ extern "C" int lbbnn_counter_inc(int64_t* counter, lbbnn_stream s) {
   LBBNN_REQUIRE(counter, "NULL counter");
   counter_inc_kernel<<<1, 1, 0, (cudaStream_t)s>>>(counter);
   return check_launch("counter_inc");
+}
+
+extern "C" int lbbnn_adam_pack_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, int64_t grad_offset,
+                                   lbbnn_stream s) {
+  LBBNN_REQUIRE(table_dev && n_entries > 0 && total_blocks > 0 && total_blocks < (1LL << 31), "bad argument");
+  adam_pack_kernel<<<(unsigned)total_blocks, 256, 0, (cudaStream_t)s>>>(table_dev, n_entries, grad_offset);
+  return check_launch("adam_pack");
+}
+
+extern "C" int lbbnn_adam_multi_dp_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t block_lo, int64_t block_hi,
+                                       const float* arena, float* arena_mc, int64_t grad_offset, float lr, float beta1,
+                                       float beta2, float eps, int64_t* step_dev, float* coef_scratch, int advance,
+                                       lbbnn_stream s) {
+  LBBNN_REQUIRE(table_dev && arena && arena_mc && step_dev && coef_scratch && n_entries > 0 && 0 <= block_lo &&
+                block_lo <= block_hi && block_hi < (1LL << 31) && grad_offset % 4 == 0 &&
+                (reinterpret_cast<uintptr_t>(arena) & 15u) == 0 && (reinterpret_cast<uintptr_t>(arena_mc) & 15u) == 0,
+                "bad argument");
+  if (advance) adam_prepare_inc<<<1, 1, 0, (cudaStream_t)s>>>(step_dev, lr, beta1, beta2, coef_scratch);
+  else adam_prepare<<<1, 1, 0, (cudaStream_t)s>>>(step_dev, lr, beta1, beta2, coef_scratch);
+  if (int rc = check_launch("adam_prepare")) return rc;
+  if (block_hi == block_lo) return LBBNN_OK;                 // more ranks than blocks: this one owns nothing
+  adam_multi_dp_kernel<<<(unsigned)(block_hi - block_lo), 256, 0, (cudaStream_t)s>>>(table_dev, n_entries, block_lo, arena, arena_mc,
+                                                                                     grad_offset, beta1, beta2, eps, coef_scratch);
+  return check_launch("adam_multi_dp");
 }

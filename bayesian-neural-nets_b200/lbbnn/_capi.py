@@ -221,6 +221,8 @@ SIGNATURES = {
     "lbbnn_adam_multi_f32": (_INT, [_P, _INT, _I64, _F, _F, _F, _F, _P, _P, _P]),
     "lbbnn_adam_multi_step_f32": (_INT, [_P, _INT, _I64, _F, _F, _F, _F, _P, _P, _P]),
     "lbbnn_nll_kl_objective_f32": (_INT, [_P, _P, _I64, _I64, _P, _P, _INT, _F, _P, _P, _P]),
+    "lbbnn_adam_pack_f32": (_INT, [_P, _INT, _I64, _I64, _P]),
+    "lbbnn_adam_multi_dp_f32": (_INT, [_P, _INT, _I64, _I64, _P, _P, _I64, _F, _F, _F, _F, _P, _P, _INT, _P]),
     "lbbnn_counter_inc": (_INT, [_P, _P]),
     "lbbnn_adamw_f32": (_INT, [_P, _P, _P, _P, _I64, _F, _F, _F, _F, _F, _P, _P, _P]),
     "lbbnn_vd_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
@@ -334,6 +336,31 @@ class graph_noise:
     def __exit__(self, *exc):
         global _graph_noise_step
         _graph_noise_step = self.prev
+
+
+# Data-parallel training (engine.GraphedTrainer with a process group): the noise that belongs to the minibatch ROWS -- the
+# activation eps of the LRT / MNF layers -- must differ between ranks, while the draws that depend on the parameters only are
+# shared.  While a trainer holds row_noise_rank(rank), lrt.py adds 0x9E3779B97F4A7C15 * rank to the seed of the activation
+# noise (the convention of the LRT trainers) and nothing else.
+_row_seed_offset = 0
+
+
+class row_noise_rank:
+    def __init__(self, rank):
+        self.offset = (0x9E3779B97F4A7C15 * int(rank)) & (2 ** 64 - 1)
+
+    def __enter__(self):
+        global _row_seed_offset
+        self.prev, _row_seed_offset = _row_seed_offset, self.offset
+        return self
+
+    def __exit__(self, *exc):
+        global _row_seed_offset
+        _row_seed_offset = self.prev
+
+
+def row_noise_seed(seed):
+    return (seed + _row_seed_offset) & (2 ** 64 - 1)
 
 
 def make_noise(eps=None, seed=0, stream_id=0, step_dev=None, step_stride=0):

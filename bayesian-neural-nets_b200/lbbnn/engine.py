@@ -26,6 +26,13 @@ def _pad4(n):
     return (n + 3) // 4 * 4
 
 
+def shard_blocks(total_blocks, world, rank):
+    """[lo, hi) of the 1024-element blocks of an Adam table that `rank` of `world` updates under the sharded data-parallel
+    update: contiguous runs of ceil(total / world) blocks, the last ranks' runs shorter or empty."""
+    per = -(-int(total_blocks) // int(world))
+    return min(total_blocks, rank * per), min(total_blocks, (rank + 1) * per)
+
+
 class LRTTrainer:
     def __init__(self, net, batch_size, num_batches, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, seed=None,
                  use_graph=True, inject_noise=False, process_group=None, fused=None, materialize_grads=True):
@@ -1181,6 +1188,85 @@ class MultiTensorAdam:
         self._late_ids, self._early_n = None, 0
         self._early_table = self._early_stream = self._early_pending = None
         self._armed, self._early_seen, self._early_events, self._early_done = False, 0, [], False
+        self.dp = None
+
+    def data_parallel(self, process_group):
+        """Data-parallel mode: the update applies the SUM over the ranks of `process_group` of every rank's gradients.
+        Parameters (re-pointed here, so modules and state_dict() keep working) and the packed gradients live in one arena
+        [parameters | packed gradients], each tensor at a 4-float aligned offset, its gradient `n_flat` floats after it;
+        the early group (set_late_params, call that first) is laid out before the late one so that each group's gradients
+        are one contiguous span.  Each update packs autograd's gradients into the arena (one launch), then
+        LBBNN_DP_UPDATE = auto (default) | sharded | nccl:
+          sharded  the arena is symmetric memory bound to an NVSwitch multicast object; between two cross-rank barriers each
+                   rank reduces (in the switch), updates and multicasts ITS contiguous 1 / world of the table's blocks
+                   (lbbnn_adam_multi_dp_f32) and keeps Adam moments for those only -- see owned_range();
+          nccl     torch.distributed.all_reduce of the group's packed gradients, then the replicated update.
+        auto takes sharded where the fabric has multicast.  Every rank must hold the same parameters (same order)."""
+        import torch.distributed as dist
+        world, rank = dist.get_world_size(process_group), dist.get_rank(process_group)
+        late = self._late_ids or set()
+        order = [p for p in self.params if id(p) not in late] + [p for p in self.params if id(p) in late]
+        scale = {id(p): sc for p, sc in zip(self.params, self.lr_scale)}
+        self.params, self.lr_scale = order, [scale[id(p)] for p in order]
+        offs, total = [], 0
+        for p in self.params:
+            offs.append(total)
+            total += _pad4(p.numel())
+        self.offs, self.n_flat = offs, total
+        dev = self.params[0].device
+        mode = os.environ.get("LBBNN_DP_UPDATE", "auto")
+        if mode not in ("auto", "sharded", "nccl"):
+            raise K.LbbnnError(f"LBBNN_DP_UPDATE={mode!r}: expected auto, sharded or nccl")
+        arena = hdl = None
+        if mode != "nccl":
+            try:
+                import torch.distributed._symmetric_memory as symm_mem
+                arena = symm_mem.empty(2 * total, dtype=torch.float32, device=dev)
+                arena.zero_()
+                hdl = symm_mem.rendezvous(arena, process_group.group_name)
+                if int(hdl.multicast_ptr) == 0:
+                    raise RuntimeError("no multicast support on this fabric")
+                hdl.barrier(channel=0)
+                torch.cuda.synchronize()
+            except Exception as e:  # noqa: BLE001
+                if mode == "sharded":
+                    raise
+                self._dp_error, arena, hdl = repr(e), None, None
+        if arena is None:
+            arena = torch.zeros(2 * total, dtype=torch.float32, device=dev)
+        with torch.no_grad():
+            for p, off in zip(self.params, offs):
+                view = arena[off:off + p.numel()].view(p.shape)
+                view.copy_(p.data)
+                p.data = view
+        early_n = len(self.params) - len(late)
+        spans = [(0, offs[early_n] if early_n < len(offs) else total), (offs[early_n] if early_n < len(offs) else total, total)]
+        self.exp_avg = torch.zeros(total, dtype=torch.float32, device=dev)
+        self.exp_avg_sq = torch.zeros(total, dtype=torch.float32, device=dev)
+        # pack rows [0, R) and, for the nccl form, the replicated update's rows (gradient = packed copy) [R, 2R)
+        self.table = torch.zeros(2 * len(self.params), 7, dtype=torch.int64, device=dev)
+        if self._late_ids is not None:
+            self._early_table = torch.zeros(2 * early_n, 7, dtype=torch.int64, device=dev)
+        self.dp = dict(pg=process_group, world=world, rank=rank, arena=arena, hdl=hdl, spans=spans, early_n=early_n,
+                       mode="sharded" if hdl is not None else "nccl",
+                       mc=int(hdl.multicast_ptr) if hdl is not None else 0)
+
+    def owned_range(self, p):
+        """Element range [lo, hi) of parameter `p` whose Adam moments (and update) THIS rank owns: all of it, except under
+        the sharded data-parallel update, where each group's table is split into contiguous runs of blocks (shard_blocks)."""
+        n = p.numel()
+        if self.dp is None or self.dp["mode"] != "sharded":
+            return 0, n
+        late = self._late_ids is not None and id(p) in self._late_ids
+        group = [q for q in self.params if (self._late_ids is not None and id(q) in self._late_ids) == late]
+        first, total = 0, sum((q.numel() + 1023) // 1024 for q in group)
+        for q in group:
+            if q is p:
+                break
+            first += (q.numel() + 1023) // 1024
+        lo, hi = shard_blocks(total, self.dp["world"], self.dp["rank"])
+        lo, hi = max(lo, first) - first, min(hi, first + (n + 1023) // 1024) - first
+        return (min(n, 1024 * lo), min(n, 1024 * hi)) if hi > lo else (0, 0)
 
     def set_late_params(self, late_params):
         """Update everything BUT `late_params` as soon as its gradients are final, in the middle of the backward: every
@@ -1221,7 +1307,7 @@ class MultiTensorAdam:
         for ev in self._early_events:
             self._early_stream.wait_event(ev)
         with torch.cuda.stream(self._early_stream):
-            self._launch(rows, blocks, self._early_table, "_early_pending", advance=True)
+            self._launch(rows, blocks, self._early_table, "_early_pending", advance=True, group=0)
         self._early_done = True
 
     def zero_grad(self, set_to_none=True):
@@ -1251,15 +1337,24 @@ class MultiTensorAdam:
             blocks += (n + 1023) // 1024
         return rows, blocks
 
-    def _launch(self, rows, blocks, table, pending_attr, advance):
+    def _table_rows(self, rows):
+        if self.dp is None:
+            return rows
+        gdist = 4 * self.n_flat            # the replicated update of the nccl form reads the packed (all-reduced) copy
+        return rows + [[r[0], r[0] + gdist] + r[2:] for r in rows]
+
+    def _launch(self, rows, blocks, table, pending_attr, advance, group=None):
+        """group (data parallel): 0 = the early group, 1 = the late group, None = every parameter."""
         if torch.cuda.is_current_stream_capturing():
             prev = getattr(self, pending_attr)
             if prev is not None and len(prev) != len(rows):
                 raise K.LbbnnError("the set of parameters with gradients changed during capture")
             setattr(self, pending_attr, rows)
         else:
-            table[:len(rows)].copy_(torch.tensor(rows, dtype=torch.int64))
+            table[:2 * len(rows) if self.dp is not None else len(rows)].copy_(torch.tensor(self._table_rows(rows), dtype=torch.int64))
         st = K.current_stream()
+        if self.dp is not None:
+            return self._launch_dp(rows, blocks, table, advance, group, st)
         if advance:                    # t_dev += 1 and the bias corrections of update t in the first of the two launches
             K.check(K.lib.lbbnn_adam_multi_step_f32(table.data_ptr(), len(rows), blocks, self.base_lr, self.betas[0],
                                                     self.betas[1], self.eps, K.ptr(self.t_dev, torch.int64), K.ptr(self.coef), st))
@@ -1277,14 +1372,41 @@ class MultiTensorAdam:
             rows, blocks = self._rows()
         if not rows:
             return
-        self._launch(rows, blocks, self.table, "_pending", advance=not early_done)
+        self._launch(rows, blocks, self.table, "_pending", advance=not early_done, group=1 if early_done else None)
+
+    def _launch_dp(self, rows, blocks, table, advance, group, st):
+        D = self.dp
+        n_group = {None: len(self.params), 0: D["early_n"], 1: len(self.params) - D["early_n"]}[group]
+        if len(rows) != n_group:
+            raise K.LbbnnError("data-parallel MultiTensorAdam: every parameter needs a gradient on every step")
+        K.check(K.lib.lbbnn_adam_pack_f32(table.data_ptr(), len(rows), blocks, self.n_flat, st))
+        tp = K.ptr(self.t_dev, torch.int64)
+        if D["mode"] == "sharded":
+            # group 0 (early, its own stream) and the late group are in flight at the same time: separate barrier channels.
+            # First barrier: every rank has packed; second: every rank's multicast stores have landed (and no rank packs
+            # the next step's gradients while a peer still reduces these)
+            ch = 1 if group == 0 else 0
+            lo, hi = shard_blocks(blocks, D["world"], D["rank"])
+            D["hdl"].barrier(channel=ch)
+            K.check(K.lib.lbbnn_adam_multi_dp_f32(table.data_ptr(), len(rows), lo, hi, D["arena"].data_ptr(), D["mc"], self.n_flat,
+                                                  self.base_lr, self.betas[0], self.betas[1], self.eps, tp, K.ptr(self.coef),
+                                                  1 if advance else 0, st))
+            D["hdl"].barrier(channel=ch)
+            return
+        a, b = D["spans"][group] if group is not None else (0, self.n_flat)
+        torch.distributed.all_reduce(D["arena"][self.n_flat + a:self.n_flat + b], group=D["pg"])
+        upd = table.data_ptr() + table.stride(0) * 8 * len(rows)
+        fn = K.lib.lbbnn_adam_multi_step_f32 if advance else K.lib.lbbnn_adam_multi_f32
+        K.check(fn(upd, len(rows), blocks, self.base_lr, self.betas[0], self.betas[1], self.eps, tp, K.ptr(self.coef), st))
 
     def finish_capture(self):
         if self._pending is not None:
-            self.table[:len(self._pending)].copy_(torch.tensor(self._pending, dtype=torch.int64))
+            rows = self._table_rows(self._pending)
+            self.table[:len(rows)].copy_(torch.tensor(rows, dtype=torch.int64))
             self._pending = None
         if self._early_pending is not None:
-            self._early_table[:len(self._early_pending)].copy_(torch.tensor(self._early_pending, dtype=torch.int64))
+            rows = self._table_rows(self._early_pending)
+            self._early_table[:len(rows)].copy_(torch.tensor(rows, dtype=torch.int64))
             self._early_pending = None
 
 
@@ -1296,15 +1418,27 @@ class GraphedTrainer:
     Reference: the body of `train` for one minibatch -- LBBNN-GP-MF-MNF.py:263-275 (objective="kl": nll_loss(sum) +
     net.kl()/NUM_BATCHES) and LBBNN-GP-MF.py:325-343 (objective="elbo": net.sample_elbo).  The eager modules run the
     same kernels one Python call at a time (~8 ms per MNF step on B200, host-bound); the replay removes the host.  The
-    optimizer is MultiTensorAdam by default: one launch instead of torch's ~40 multi_tensor_apply launches per step."""
+    optimizer is MultiTensorAdam by default: one launch instead of torch's ~40 multi_tensor_apply launches per step.
+
+    Data parallel (process_group): each rank runs the captured step on its own `batch_size` rows of the minibatch and the
+    optimizer applies the SUM over ranks of the gradients (the nll is a sum over rows, MNF:267-270 / MF:308), so the step
+    is the single-GPU step on the concatenated minibatch.  The draws that depend on the parameters only -- MNF's z draw and
+    flow masks and its KL branch's draws, MF's masks, sampled weights, bias noise and Gamma precisions -- are ONE draw per
+    step for the whole minibatch in the reference, so every rank makes the same draw (same lbbnn / torch seeds, same
+    modules built in the same order: checked at construction); the per-row activation noise of the LRT / MNF layers is
+    disjoint across ranks (seed + 0x9E3779B97F4A7C15 * rank); the replicated scalar terms (MNF's kl, MF's log q and
+    log prior) enter each rank's objective at 1 / world, so their gradient is counted once.  Rank 0's parameters are
+    broadcast at construction; MultiTensorAdam.data_parallel does the exchange."""
 
     def __init__(self, net, batch_size, num_batches, objective="kl", lr=1e-3, betas=(0.9, 0.999), eps=1e-8,
-                 in_features=None, optimizer=None, param_groups=None, fuse_objective=True):
+                 in_features=None, optimizer=None, param_groups=None, fuse_objective=True, process_group=None):
         """optimizer: None = MultiTensorAdam (one launch for all parameters); "torch" = torch.optim.Adam(capturable=True);
         or any capturable torch optimizer instance over net.parameters().
         param_groups: torch.optim-style parameter groups with their own learning rates (the MF script's 33 groups,
         MF:520-553: `lbbnn.mf.reference_param_groups(net)`), for the first two optimizer choices.
-        fuse_objective: objective="kl" through the one-launch loss head (_fused_objective) where the network allows it."""
+        fuse_objective: objective="kl" through the one-launch loss head (_fused_objective) where the network allows it.
+        process_group: data-parallel training over the ranks of this torch.distributed group (see the class docstring);
+        needs optimizer=None.  batch_size is the rows of ONE rank."""
         K.require_device()
         self.net, self.B, self.num_batches, self.objective = net, int(batch_size), num_batches, objective
         params = list(net.parameters())
@@ -1312,6 +1446,13 @@ class GraphedTrainer:
         if dev.type != "cuda":
             raise K.LbbnnError("GraphedTrainer needs the network on a CUDA device (no CPU fallback)")
         self.device = dev
+        self.pg = process_group
+        self.world = 1 if process_group is None else torch.distributed.get_world_size(process_group)
+        self.rank = 0 if process_group is None else torch.distributed.get_rank(process_group)
+        if process_group is not None:
+            if optimizer is not None:
+                raise K.LbbnnError("data-parallel GraphedTrainer runs the built-in MultiTensorAdam only (optimizer=None)")
+            self._check_replicas(params)
         in_features = in_features or net.sizes[0]
         self.x = torch.zeros(self.B, in_features, dtype=torch.float32, device=dev)
         self.y = torch.zeros(self.B, dtype=torch.int64, device=dev)
@@ -1320,6 +1461,8 @@ class GraphedTrainer:
             self.opt = MultiTensorAdam(param_groups if param_groups is not None else params, lr=lr, betas=betas, eps=eps)
             if hasattr(net, "late_grad_params") and os.environ.get("LBBNN_ADAM_SPLIT", "1") == "1":
                 self.opt.set_late_params(net.late_grad_params())
+            if process_group is not None:
+                self.opt.data_parallel(process_group)
         elif isinstance(optimizer, str) and optimizer == "torch":
             self.opt = torch.optim.Adam(param_groups if param_groups is not None else params, lr=lr, betas=betas, eps=eps,
                                         capturable=True)
@@ -1334,18 +1477,33 @@ class GraphedTrainer:
         net.train()
         self._stream = torch.cuda.Stream(device=dev)
         self._stream.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(self._stream), K.graph_noise(self.step_dev):
+        with torch.cuda.stream(self._stream), K.graph_noise(self.step_dev), K.row_noise_rank(self.rank):
             for _ in range(3):                      # warm-up: sizes every workspace, creates the Adam state
                 self._one_step()
         torch.cuda.current_stream().wait_stream(self._stream)
         torch.cuda.synchronize()
         self.opt.zero_grad(set_to_none=True)        # gradients are re-allocated from the graph's private pool
         self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph, stream=self._stream), K.graph_noise(self.step_dev):
+        with torch.cuda.graph(self.graph, stream=self._stream), K.graph_noise(self.step_dev), K.row_noise_rank(self.rank):
             self._one_step()
         if isinstance(self.opt, MultiTensorAdam):
             self.opt.finish_capture()
         self.warmup_steps = 3
+
+    def _check_replicas(self, params):
+        """Every rank must make the same parameter-side draws: same lbbnn and torch CUDA seeds (checked), same modules
+        in the same order (the parameter shapes are checked); then rank 0's parameters are broadcast."""
+        import torch.distributed as dist
+        mine = (_lrt.current_seed(), torch.cuda.initial_seed(), [tuple(p.shape) for p in params])
+        allv = [None] * self.world
+        dist.all_gather_object(allv, mine, group=self.pg)
+        if any(v != allv[0] for v in allv):
+            raise K.LbbnnError("data-parallel GraphedTrainer: ranks differ in lbbnn.manual_seed / torch.manual_seed or in the "
+                               "network (seed, torch seed, parameter shapes per rank: %r)" % ([v[:2] for v in allv],))
+        src = dist.get_global_rank(self.pg, 0)
+        with torch.no_grad():
+            for p in params:
+                dist.broadcast(p.data, src=src, group=self.pg)
 
     def _fused_objective(self):
         """The objective through ONE launch (lbbnn_nll_kl_objective_f32) where the network exposes its logits and its
@@ -1371,11 +1529,12 @@ class GraphedTrainer:
             raise K.LbbnnError("fused objective: the network's logits / scalar terms are not what the kernel takes")
         if self._dlogits is None or self._dlogits.shape != logits.shape:
             self._dlogits = torch.empty_like(logits)
-            self._kl_grads = [torch.full_like(k, sg / self.num_batches) for k, sg in zip(terms, signs)]    # d loss / d term_i
+            # d loss / d term_i; data parallel: the terms are replicated, each rank takes them at 1 / world
+            self._kl_grads = [torch.full_like(k, sg / (self.num_batches * self.world)) for k, sg in zip(terms, signs)]
         ptrs = (C_void_p * len(terms))(*[k.data_ptr() for k in terms])
         scales = (C_float * len(terms))(*signs)
         K.check(K.lib.lbbnn_nll_kl_objective_f32(K.ptr(logits), K.ptr(self.y, torch.int64), logits.shape[0], logits.shape[1],
-                                                 ptrs, scales, len(terms), 1.0 / self.num_batches, K.ptr(self.stats),
+                                                 ptrs, scales, len(terms), 1.0 / (self.num_batches * self.world), K.ptr(self.stats),
                                                  K.ptr(self._dlogits), K.current_stream()))
         torch.autograd.backward([logits] + terms, [self._dlogits] + self._kl_grads)
         return True
@@ -1388,10 +1547,12 @@ class GraphedTrainer:
             if self.objective == "elbo":
                 out = self.net.sample_elbo(self.x, self.y)
                 loss, nll = out[0], out[3]
+                if self.world > 1:         # loss = nll + (log q - log prior) / num_batches with the replicated terms at 1 / world
+                    loss = nll + (out[2] - out[1]) / (self.net.num_batches * self.world)
             else:
                 logp = self.net(self.x, sample=True)
                 nll = torch.nn.functional.nll_loss(logp, self.y, reduction="sum")
-                loss = nll + self.net.kl() / self.num_batches
+                loss = nll + self.net.kl() / (self.num_batches * self.world)
             loss.backward()
             self.opt.step()
             self.stats.copy_(torch.stack([loss.detach(), nll.detach()]))
@@ -1418,6 +1579,8 @@ class GraphedTrainer:
         return self._stats_dict(self.stats_host)
 
     def _stats_dict(self, st):
+        """[loss, nll] of the step.  Data parallel: THIS RANK's contribution (its rows' nll, the replicated terms at
+        1 / world); the sum over ranks is the single-GPU value of the concatenated minibatch."""
         return {"loss": float(st[0]), "nll": float(st[1])}
 
     # the pipelined host-buffer step of the LRT trainers: upload of batch i+1 on a copy stream under step i, the [loss, nll]

@@ -73,7 +73,7 @@ class _LRTFunction(torch.autograd.Function):
             eps = eps.contiguous()
             if tuple(eps.shape) != (B, out_f):
                 raise K.LbbnnError(f"eps must be {(B, out_f)}, got {tuple(eps.shape)}")
-        noise = K.make_noise(eps, noise_key[0], noise_key[1])
+        noise = K.make_noise(eps, K.row_noise_seed(noise_key[0]), noise_key[1])    # per-row noise: disjoint across ranks
         flags = (K.FLAG_SAMPLE if sample else 0) | (K.FLAG_KL if want_kl else 0) | (K.FLAG_RELU if relu else 0)
         act = torch.empty(B, out_f, dtype=torch.float32, device=x.device)
         dsf = torch.empty(B, out_f, dtype=torch.float32, device=x.device) if sample else None

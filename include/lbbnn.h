@@ -655,6 +655,23 @@ LBBNN_API int lbbnn_adam_multi_f32(const lbbnn_adam_entry* table_dev, int n_entr
 LBBNN_API int lbbnn_adam_multi_step_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, float lr,
                                         float beta1, float beta2, float eps, int64_t* step_dev, float* coef_scratch,
                                         lbbnn_stream s);
+/* Data-parallel form of the table update above, for the training step of LBBNN-GP-MF-MNF.py:263-275 and
+ * LBBNN-GP-MF.py:325-343 with the minibatch sharded over ranks: torch.optim.Adam of the SUM over ranks of the gradients.
+ * Every entry's param lies in one symmetric-memory arena [parameters | packed gradients] that is bound to an NVSwitch
+ * multicast object (arena_mc is its multicast address), each tensor at a 16-byte aligned offset and padded with zeros to a
+ * multiple of 4 floats; its packed gradient sits grad_offset floats (a multiple of 4) after it.
+ *   pack:  param[grad_offset + i] = grad[i] for every entry -- this rank's gradients into its region of the arena.
+ *   dp:    blocks [block_lo, block_hi) of the table (one rank's share, 1024 elements each; the ranks' shares cover every
+ *          block once): in-switch sum over ranks of the packed gradient (multimem.ld_reduce), Adam on this rank's exp_avg /
+ *          exp_avg_sq with lr * lr_scale, the new parameter stored to every rank's arena (multimem.st).  advance != 0:
+ *          *step_dev += 1 first, as lbbnn_adam_multi_step_f32; 0: as lbbnn_adam_multi_f32.
+ * The caller orders the dp launch between two cross-rank barriers: every rank packed before, every store landed after. */
+LBBNN_API int lbbnn_adam_pack_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, int64_t grad_offset,
+                                  lbbnn_stream s);
+LBBNN_API int lbbnn_adam_multi_dp_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t block_lo, int64_t block_hi,
+                                      const float* arena, float* arena_mc, int64_t grad_offset, float lr, float beta1,
+                                      float beta2, float eps, int64_t* step_dev, float* coef_scratch, int advance,
+                                      lbbnn_stream s);
 LBBNN_API int lbbnn_counter_inc(int64_t* counter, lbbnn_stream s);
 /* torch.optim.AdamW (variational_dropout.py:110): the update above preceded by param *= 1 - lr * weight_decay */
 LBBNN_API int lbbnn_adamw_f32(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,

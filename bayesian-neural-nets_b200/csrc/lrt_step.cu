@@ -1492,19 +1492,27 @@ double mac_clk(const TileCfg& c) {
 double stage_clk(double float4_units) { return 600.0 + 450.0 * float4_units / NT; }
 double reduce_clk(const TileCfg& c) { return (c.G > 1 ? 1000.0 + 450.0 * (c.G - 1) : 0.0) + 1500.0; }
 
-bool env_plan(int l, int v[6]) {
+// LBBNN_STEP_PLAN_L<l> = "bn,fsplits,rn,ck,bk,xsplits" forces layer l's forward column tile and split count, dW tile and
+// dX column tile and split count (0 = left to the cost model; layer 0 has no dX phase).  v = all zeros when unset.
+int env_plan(int l, int v[6]) {
   char name[64];
   snprintf(name, sizeof(name), "LBBNN_STEP_PLAN_L%d", l);
-  const char* s = getenv(name);
-  if (!s) return false;
   for (int i = 0; i < 6; ++i) v[i] = 0;
-  sscanf(s, "%d,%d,%d,%d,%d,%d", &v[0], &v[1], &v[2], &v[3], &v[4], &v[5]);
-  return true;
+  const char* s = getenv(name);
+  if (!s) return LBBNN_OK;
+  int end = -1;
+  const int got = sscanf(s, "%d,%d,%d,%d,%d,%d%n", &v[0], &v[1], &v[2], &v[3], &v[4], &v[5], &end);
+  bool ok = got == 6 && end >= 0 && s[end] == '\0';
+  for (int i = 0; i < 6; ++i) ok = ok && v[i] >= 0;
+  LBBNN_REQUIRE(ok, "%s=\"%s\": expected bn,fsplits,rn,ck,bk,xsplits (integers >= 0, 0 = free)", name, s);
+  LBBNN_REQUIRE(l > 0 || (v[4] == 0 && v[5] == 0), "%s=\"%s\": layer 0 has no dX phase, bk and xsplits must be 0", name, s);
+  return LBBNN_OK;
 }
 
-int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out);
+int plan_step_uncached(const lbbnn_step* S, int G, const int (*ov)[6], bool generic_head, HostPlan* out);
 
-// The schedule search costs ~1 ms; cache it per (batch, shapes, var_modes, G) so eager (non-graph) steps do not pay it.
+// The schedule search costs ~1 ms; cache it per (G, batch, shapes, overrides) so eager (non-graph) steps do not pay it.
+// The overrides are part of the key: setting or clearing one replans.
 int plan_step(const lbbnn_step* S, int G, HostPlan* out) {
   static std::mutex mu;
   static std::vector<int64_t> cached_key;
@@ -1512,14 +1520,19 @@ int plan_step(const lbbnn_step* S, int G, HostPlan* out) {
   LBBNN_REQUIRE(S != nullptr, "step is NULL");
   std::vector<int64_t> key = {G, S->n_layers, S->batch};
   const bool sane = S->n_layers >= 1 && S->n_layers <= kMaxL;
+  int ov[kMaxL][6] = {};
   for (int l = 0; sane && l < S->n_layers; ++l) {
     key.push_back(S->layer[l].in_features);
     key.push_back(S->layer[l].out_features);
+    if (int rc = env_plan(l, ov[l])) return rc;
+    key.insert(key.end(), ov[l], ov[l] + 6);
   }
+  const bool generic_head = getenv("LBBNN_STEP_GENERIC_HEAD") != nullptr;
+  key.push_back(generic_head);
   std::lock_guard<std::mutex> lock(mu);
   if (!sane || key != cached_key) {
     HostPlan P;
-    if (int rc = plan_step_uncached(S, G, &P)) return rc;
+    if (int rc = plan_step_uncached(S, G, ov, generic_head, &P)) return rc;
     cached = P;
     cached_key = key;
   }
@@ -1537,7 +1550,7 @@ int plan_step(const lbbnn_step* S, int G, HostPlan* out) {
   return LBBNN_OK;
 }
 
-int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
+int plan_step_uncached(const lbbnn_step* S, int G, const int (*ovr)[6], bool generic_head, HostPlan* out) {
   LBBNN_REQUIRE(S != nullptr, "step is NULL");
   LBBNN_REQUIRE(S->n_layers >= 1 && S->n_layers <= kMaxL, "n_layers must be 1..%d", kMaxL);
   LBBNN_REQUIRE(S->batch >= 1 && S->batch <= 128, "the fused step kernel handles batch <= 128 (got %lld)", (long long)S->batch);
@@ -1565,22 +1578,22 @@ int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
     y.off_bmu = s.off_bias_mu; y.off_brho = s.off_bias_rho;
     y.eps = s.eps; y.pri = s.priors; y.var_mode = s.var_mode;
     const int K = y.K, N = y.N;
-    int ov[6] = {0, 0, 0, 0, 0, 0};
-    const bool has_ov = env_plan(l, ov);
+    const int* ov = ovr[l];
+    const bool forced = ov[0] || ov[1] || ov[2] || ov[3] || ov[4] || ov[5];
     auto red_floats = [](const TileCfg& c) {
       return (size_t)(c.G <= 1 ? 0 : (c.G <= 8 ? c.G - 1 : (c.G + 1) / 2)) * 64 * c.TPG;
     };
     // ---- forward: column tile bn x contraction splits ----
     double best = 1e300;
     for (int bn : kBn) {
-      if (has_ov && ov[0] && bn != ov[0]) continue;
+      if (ov[0] && bn != ov[0]) continue;
       const int bnc = std::min(bn, r8(N));
       const int Cc = std::min(bnc, N);
       if (RGB * (r8(Cc) / 8) > NT) continue;
       const int ntiles = cdiv(N, bnc);
       const int max_splits = std::max(1, std::min(G / std::max(1, std::min(ntiles, G)), cdiv(K, 8)));
       for (int sp = 1; sp <= max_splits; ++sp) {
-        if (has_ov && ov[1] && sp != ov[1]) continue;
+        if (ov[1] && sp != ov[1]) continue;
         const int kc = r4(cdiv(K, sp));
         const int s2 = cdiv(K, kc);
         const TileCfg c = make_cfg(B, Cc, kc, NT);
@@ -1597,16 +1610,17 @@ int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
         }
       }
     }
-    LBBNN_REQUIRE(best < 1e300, "no forward schedule fits layer %d (%d -> %d) in shared memory", l, K, N);
+    LBBNN_REQUIRE(best < 1e300, "no forward schedule fits layer %d (%d -> %d) in shared memory%s", l, K, N,
+                  forced ? " under the forced LBBNN_STEP_PLAN_L values" : "");
     part_floats = std::max(part_floats, (size_t)y.f_splits * 2 * B * N);
     // ---- backward: dW tiles (rn x ck) and dX tiles (bk columns x contraction splits) share a phase ----
     best = 1e300;
     for (int rn : kRn) {
-      if (has_ov && ov[2] && rn != ov[2]) continue;
+      if (ov[2] && rn != ov[2]) continue;
       const int rnc = std::min(rn, r4(N));
       const int Rw = std::min(rnc, N);
       for (int ck : kCk) {
-        if (has_ov && ov[3] && ck != ov[3]) continue;
+        if (ov[3] && ck != ov[3]) continue;
         const int ckc = std::min(ck, r8(K));
         const int Cw = std::min(ckc, K);
         if ((r4(Rw) / 4) * (r8(Cw) / 8) > NT) continue;
@@ -1617,14 +1631,14 @@ int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
         const int nbk = l > 0 ? (int)(sizeof(kBk) / sizeof(int)) : 1;
         for (int bi = 0; bi < nbk; ++bi) {
           const int bk = kBk[bi];
-          if (l > 0 && has_ov && ov[4] && bk != ov[4]) continue;
+          if (ov[4] && bk != ov[4]) continue;
           const int bkc = std::min(bk, r8(K));
           const int Cx = std::min(bkc, K);
           if (l > 0 && RGB * (r8(Cx) / 8) > NT) continue;
           const int xct = cdiv(K, bkc);
           const int max_sp = l > 0 ? std::max(1, std::min(cdiv(N, 4), G)) : 1;
           for (int sp = 1; sp <= max_sp; ++sp) {
-            if (l > 0 && has_ov && ov[5] && sp != ov[5]) continue;
+            if (ov[5] && sp != ov[5]) continue;
             const int nc = r4(cdiv(N, sp));
             const int s2 = cdiv(N, nc);
             if (s2 != sp && sp > 1) continue;
@@ -1648,7 +1662,8 @@ int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
         }
       }
     }
-    LBBNN_REQUIRE(best < 1e300, "no backward schedule fits layer %d (%d -> %d) in shared memory", l, K, N);
+    LBBNN_REQUIRE(best < 1e300, "no backward schedule fits layer %d (%d -> %d) in shared memory%s", l, K, N,
+                  forced ? " under the forced LBBNN_STEP_PLAN_L values" : "");
     y.fc = make_cfg(B, std::min(y.f_bn, N), y.f_kc, NT);
     y.wc = make_cfg(std::min(y.w_rn, N), std::min(y.w_ck, K), B, NT);
     y.xc = make_cfg(B, std::min(y.x_bk, K), y.x_nc, NT);
@@ -1660,7 +1675,7 @@ int plan_step_uncached(const lbbnn_step* S, int G, HostPlan* out) {
   {
     const int Nl = d.ly[d.L - 1].N;
     d.small_last = (Nl <= 32 && cdiv(B, d.nll_ctas) <= NT / 32 && 2 * B * Nl + 32 * B <= kWOff &&
-                    !getenv("LBBNN_STEP_GENERIC_HEAD")) ? 1 : 0;
+                    !generic_head) ? 1 : 0;
   }
   LBBNN_REQUIRE(d.nll_ctas <= G, "batch too large for the loss phase");
   P.smem = smem;
@@ -1800,7 +1815,8 @@ extern "C" int lbbnn_lrt_step_f32(const lbbnn_step* S, int phases, void* ws, siz
   return check_launch("lrt_step_kernel");
 }
 
-// schedule dump for logs / DESIGN.md: "l0 F bn=.. splits=.. | W rn x ck (items) | X bk x splits (items)"
+// schedule dump for logs / DESIGN.md: "l0 F bn=.. splits=.. | W rn x ck (items) | X bk x splits (items); ... head=small|tiled smem=.."
+// (head=small: the last layer runs last_fwd_loss / last_bwd, and its F / W / X entries are not used)
 extern "C" int lbbnn_lrt_step_describe(const lbbnn_step* S, char* buf, size_t buf_bytes) {
   HostPlan P;
   if (int rc = plan_step(S, sm_count() * kCtasPerSm, &P)) return rc;
@@ -1811,6 +1827,6 @@ extern "C" int lbbnn_lrt_step_describe(const lbbnn_step* S, char* buf, size_t bu
                   y.f_bn, y.f_kc, y.f_ntiles, y.f_splits, y.w_rn, y.w_ck, y.w_rtiles * y.w_ctiles, y.x_bk, y.x_nc,
                   l > 0 ? y.x_ctiles : 0, l > 0 ? y.x_splits : 0);
   }
-  if (o < buf_bytes) snprintf(buf + o, buf_bytes - o, "smem=%zu", P.smem);
+  if (o < buf_bytes) snprintf(buf + o, buf_bytes - o, "head=%s smem=%zu", P.d.small_last ? "small" : "tiled", P.smem);
   return LBBNN_OK;
 }

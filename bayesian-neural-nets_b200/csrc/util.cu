@@ -311,6 +311,7 @@ __global__ void __launch_bounds__(256) adam_multi_kernel(const lbbnn_adam_entry*
   const float inv_bc2 = 1.0f / bc2_sqrt;
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
+    if (e.decay != 0.f) pv[j] *= 1.0f - e.decay;     // torch.optim.AdamW: param.mul_(1 - lr * weight_decay) first
     mv[j] = mv[j] + (gv[j] - mv[j]) * (1.0f - b1);
     vv[j] = b2 * vv[j] + (1.0f - b2) * gv[j] * gv[j];
     const float denom = fmaf(sqrtf(vv[j]), inv_bc2, eps);
@@ -370,6 +371,7 @@ __global__ void __launch_bounds__(256) adam_multi_dp_kernel(const lbbnn_adam_ent
   const float inv_bc2 = 1.0f / bc2_sqrt;
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
+    if (e.decay != 0.f) pv[j] *= 1.0f - e.decay;     // torch.optim.AdamW: param.mul_(1 - lr * weight_decay) first
     mv[j] = mv[j] + (gv[j] - mv[j]) * (1.0f - b1);
     vv[j] = b2 * vv[j] + (1.0f - b2) * gv[j] * gv[j];
     const float denom = fmaf(sqrtf(vv[j]), inv_bc2, eps);

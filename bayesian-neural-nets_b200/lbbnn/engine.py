@@ -33,6 +33,23 @@ def shard_blocks(total_blocks, world, rank):
     return min(total_blocks, rank * per), min(total_blocks, (rank + 1) * per)
 
 
+def check_replicas(process_group, params, what):
+    """Start of data-parallel training: every rank must make the same parameter-side draws -- same lbbnn and torch CUDA
+    seeds (checked), same modules in the same order (the parameter shapes are checked); then rank 0's parameters are
+    broadcast.  Raises LbbnnError naming `what` on a mismatch."""
+    import torch.distributed as dist
+    mine = (_lrt.current_seed(), torch.cuda.initial_seed(), [tuple(p.shape) for p in params])
+    allv = [None] * dist.get_world_size(process_group)
+    dist.all_gather_object(allv, mine, group=process_group)
+    if any(v != allv[0] for v in allv):
+        raise K.LbbnnError("%s: ranks differ in lbbnn.manual_seed / torch.manual_seed or in the network (seed, torch seed, "
+                           "parameter shapes per rank: %r)" % (what, [v[:2] for v in allv]))
+    src = dist.get_global_rank(process_group, 0)
+    with torch.no_grad():
+        for p in params:
+            dist.broadcast(p.data, src=src, group=process_group)
+
+
 class LRTTrainer:
     def __init__(self, net, batch_size, num_batches, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, seed=None,
                  use_graph=True, inject_noise=False, process_group=None, fused=None, materialize_grads=True):
@@ -334,15 +351,21 @@ class LRTTrainer:
 
     def _capture(self):
         # side stream warm-up (also sizes nothing: all buffers are preallocated), then capture
-        state = [t.clone() for t in (self.flat, self.exp_avg, self.exp_avg_sq, self.step_dev)]
+        tensors = self._train_state() if hasattr(self, "_train_state") else (self.flat, self.exp_avg, self.exp_avg_sq,
+                                                                             self.step_dev)
+        state = [t.clone() for t in tensors]
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
             self._enqueue()
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize()
-        for t, saved in zip((self.flat, self.exp_avg, self.exp_avg_sq, self.step_dev), state):
+        for t, saved in zip(tensors, state):
             t.copy_(saved)   # the warm-up step must not count as training
+        if getattr(self, "pg", None) is not None and hasattr(self, "_train_state"):
+            # data-parallel update: a peer's replay writes this rank's parameters, so no rank may replay before all restored
+            torch.cuda.synchronize()
+            torch.distributed.barrier(group=self.pg)
         if hasattr(self, "_after_restore"):
             self._after_restore()   # state derived from the parameters (carried bf16 operands)
         self.graph = torch.cuda.CUDAGraph()
@@ -1143,20 +1166,23 @@ class LRTTensorCoreTrainer:
 
 
 class MultiTensorAdam:
-    """torch.optim.Adam(params, lr, betas, eps) (non-amsgrad, no weight decay) as ONE launch over the whole parameter list
-    (lbbnn_adam_multi_f32): a device table names every (param, grad, exp_avg, exp_avg_sq, lr) record.  `params` is what
-    torch.optim takes: an iterable of tensors (MNF:352) or of parameter-group dicts {"params": ..., "lr": ...} -- the MF
-    script's 33 groups with learning rates from 1e-5 to 0.1 (MF:520-553; `lbbnn.mf.reference_param_groups(net)`).  A
-    group without "lr" uses the optimizer's.  Gradient addresses are whatever autograd produced for this step: eager steps
-    rewrite the table every call; under CUDA-graph capture the addresses (stable in the graph's private pool) are recorded
-    and the table is written once after the capture (`finish_capture`)."""
+    """torch.optim.Adam(params, lr, betas, eps) (non-amsgrad) as ONE launch over the whole parameter list
+    (lbbnn_adam_multi_f32): a device table names every (param, grad, exp_avg, exp_avg_sq, lr, decay) record.  `params` is
+    what torch.optim takes: an iterable of tensors (MNF:352) or of parameter-group dicts {"params": ..., "lr": ...,
+    "weight_decay": ...} -- the MF script's 33 groups with learning rates from 1e-5 to 0.1 (MF:520-553;
+    `lbbnn.mf.reference_param_groups(net)`).  A group without "lr" / "weight_decay" uses the optimizer's.  A non-zero
+    weight_decay makes that group's update torch.optim.AdamW's (decoupled: param *= 1 - lr * weight_decay first,
+    variational_dropout.py:110); 0 (the default) is torch.optim.Adam exactly.  Gradient addresses are whatever autograd
+    produced for this step: eager steps rewrite the table every call; under CUDA-graph capture the addresses (stable in the
+    graph's private pool) are recorded and the table is written once after the capture (`finish_capture`)."""
 
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8):
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
         self.lr, self.betas, self.eps = float(lr), (float(betas[0]), float(betas[1])), float(eps)
+        self.weight_decay = float(weight_decay)
         params = list(params)
         groups = params if (params and isinstance(params[0], dict)) else [{"params": params}]
         self.param_groups = []
-        self.params, self.lr_scale = [], []
+        self.params, self.lr_scale, self.decay = [], [], []
         seen = set()
         # the launch takes ONE base learning rate (bias correction folded in on the device); groups carry a factor
         lrs = [float(g.get("lr", self.lr)) for g in groups]
@@ -1164,7 +1190,8 @@ class MultiTensorAdam:
         for g, glr in zip(groups, lrs):
             ps = g["params"]
             ps = [ps] if torch.is_tensor(ps) else list(ps)
-            self.param_groups.append({"params": ps, "lr": glr})
+            gwd = float(g.get("weight_decay", self.weight_decay))
+            self.param_groups.append({"params": ps, "lr": glr, "weight_decay": gwd})
             for p in ps:
                 if id(p) in seen:
                     raise ValueError("some parameters appear in more than one parameter group")
@@ -1172,6 +1199,7 @@ class MultiTensorAdam:
                 if p.requires_grad:
                     self.params.append(p)
                     self.lr_scale.append(glr / self.base_lr)
+                    self.decay.append(glr * gwd)       # the table's decay: lr and weight decay are constant per group
         dev = self.params[0].device
         offs, total = [], 0
         for p in self.params:
@@ -1206,8 +1234,8 @@ class MultiTensorAdam:
         world, rank = dist.get_world_size(process_group), dist.get_rank(process_group)
         late = self._late_ids or set()
         order = [p for p in self.params if id(p) not in late] + [p for p in self.params if id(p) in late]
-        scale = {id(p): sc for p, sc in zip(self.params, self.lr_scale)}
-        self.params, self.lr_scale = order, [scale[id(p)] for p in order]
+        scale = {id(p): (sc, dc) for p, sc, dc in zip(self.params, self.lr_scale, self.decay)}
+        self.params, self.lr_scale, self.decay = order, [scale[id(p)][0] for p in order], [scale[id(p)][1] for p in order]
         offs, total = [], 0
         for p in self.params:
             offs.append(total)
@@ -1324,14 +1352,14 @@ class MultiTensorAdam:
     def _rows(self, keep=None):
         import struct
         rows, blocks = [], 0
-        for p, off, sc in zip(self.params, self.offs, self.lr_scale):
+        for p, off, sc, dc in zip(self.params, self.offs, self.lr_scale, self.decay):
             g = p.grad
             if g is None or (keep is not None and not keep(p)):
                 continue
             if g.dtype != torch.float32 or not g.is_contiguous() or not p.is_contiguous():
                 raise K.LbbnnError("MultiTensorAdam needs contiguous fp32 parameters and gradients")
             n = p.numel()
-            lr_bits = struct.unpack("<q", struct.pack("<ff", sc, 0.0))[0]       # {float lr_scale; float reserved}
+            lr_bits = struct.unpack("<q", struct.pack("<ff", sc, dc))[0]        # {float lr_scale; float decay}
             rows.append([p.data_ptr(), g.data_ptr(), self.exp_avg.data_ptr() + 4 * off,
                          self.exp_avg_sq.data_ptr() + 4 * off, n, blocks, lr_bits])
             blocks += (n + 1023) // 1024
@@ -1452,7 +1480,7 @@ class GraphedTrainer:
         if process_group is not None:
             if optimizer is not None:
                 raise K.LbbnnError("data-parallel GraphedTrainer runs the built-in MultiTensorAdam only (optimizer=None)")
-            self._check_replicas(params)
+            check_replicas(process_group, params, "data-parallel GraphedTrainer")
         in_features = in_features or net.sizes[0]
         self.x = torch.zeros(self.B, in_features, dtype=torch.float32, device=dev)
         self.y = torch.zeros(self.B, dtype=torch.int64, device=dev)
@@ -1489,21 +1517,6 @@ class GraphedTrainer:
         if isinstance(self.opt, MultiTensorAdam):
             self.opt.finish_capture()
         self.warmup_steps = 3
-
-    def _check_replicas(self, params):
-        """Every rank must make the same parameter-side draws: same lbbnn and torch CUDA seeds (checked), same modules
-        in the same order (the parameter shapes are checked); then rank 0's parameters are broadcast."""
-        import torch.distributed as dist
-        mine = (_lrt.current_seed(), torch.cuda.initial_seed(), [tuple(p.shape) for p in params])
-        allv = [None] * self.world
-        dist.all_gather_object(allv, mine, group=self.pg)
-        if any(v != allv[0] for v in allv):
-            raise K.LbbnnError("data-parallel GraphedTrainer: ranks differ in lbbnn.manual_seed / torch.manual_seed or in the "
-                               "network (seed, torch seed, parameter shapes per rank: %r)" % ([v[:2] for v in allv],))
-        src = dist.get_global_rank(self.pg, 0)
-        with torch.no_grad():
-            for p in params:
-                dist.broadcast(p.data, src=src, group=self.pg)
 
     def _fused_objective(self):
         """The objective through ONE launch (lbbnn_nll_kl_objective_f32) where the network exposes its logits and its

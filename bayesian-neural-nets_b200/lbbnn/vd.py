@@ -15,7 +15,7 @@ import torch.nn.functional as F
 
 from . import _capi as K
 from . import lrt as _lrt
-from .engine import LRTTrainer
+from .engine import LRTTrainer, MultiTensorAdam, check_replicas
 
 _layer_ids = itertools.count(1)
 
@@ -176,10 +176,20 @@ class VDTrainer:
     captured once in a CUDA graph: per layer lbbnn_vd_fwd with the relu fused in, the log-softmax / nll head,
     lbbnn_vd_bwd per layer (relu mask folded into the gradient staging), ONE AdamW launch over the flat theta buffer.
     alpha is constant unless the model was built with alpha_trainable=True (then its KL gradient is added and it is
-    updated by the same AdamW rule).  stats = [nll, kl]."""
+    updated by the same AdamW rule).  stats = [nll, kl].
+
+    Data parallel (process_group): each rank runs the captured step on its own `batch_size` rows of the minibatch and the
+    update applies the SUM over ranks of the gradients (the nll is a sum over rows, VD:104-106), so the step is the
+    single-GPU step on the concatenated minibatch.  Each rank draws its zeta from seed + 0x9E3779B97F4A7C15 * rank (the
+    rows' noise is disjoint); the KL term is replicated, so its alpha gradient enters each rank at 1 / (num_batches * world).
+    The ranks must be built alike (same seeds and shapes: checked), rank 0's parameters are broadcast, and every rank must
+    replay the same number of steps: the update is MultiTensorAdam(weight_decay=).data_parallel -- the sharded multicast
+    exchange, or the NCCL all-reduce under LBBNN_DP_UPDATE=nccl or without multicast (`dp_update` says which)."""
 
     def __init__(self, model, batch_size, num_batches=600.0, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2,
-                 seed=None, use_graph=True, inject_noise=False):
+                 seed=None, use_graph=True, inject_noise=False, process_group=None):
+        """process_group: data-parallel training over the ranks of this torch.distributed group (see the class docstring);
+        batch_size is the rows of ONE rank."""
         K.require_device()
         self.net = model
         self.layers = list(model.layers)
@@ -187,26 +197,42 @@ class VDTrainer:
         self.num_batches = float(num_batches)
         self.lr, self.betas, self.eps, self.wd = float(lr), betas, float(eps), float(weight_decay)
         self.seed = _lrt.current_seed() if seed is None else int(seed)
+        self.pg = process_group
+        self.world = 1 if process_group is None else torch.distributed.get_world_size(process_group)
+        self.rank = 0 if process_group is None else torch.distributed.get_rank(process_group)
         dev = self.layers[0].theta.device
         self.device = dev
         f32 = dict(dtype=torch.float32, device=dev)
         self.train_alpha = isinstance(self.layers[0].alpha, nn.Parameter)
+        names = ("theta", "alpha") if self.train_alpha else ("theta",)
+        if process_group is not None:
+            check_replicas(process_group, [getattr(l, n) for l in self.layers for n in names], "data-parallel VDTrainer")
         offs, total = [], 0
         for l in self.layers:
-            for name in (("theta", "alpha") if self.train_alpha else ("theta",)):
+            for name in names:
                 p = getattr(l, name)
                 offs.append((l, name, total, p.numel(), p.shape))
                 total += (p.numel() + 3) // 4 * 4
         self.n_flat = total
-        self.flat, self.gflat = torch.zeros(total, **f32), torch.zeros(total, **f32)
-        self.exp_avg, self.exp_avg_sq = torch.zeros(total, **f32), torch.zeros(total, **f32)
+        self.gflat = torch.zeros(total, **f32)
+        self.opt, self.dp_update = None, None
+        if process_group is None:
+            self.flat = torch.zeros(total, **f32)
+            self.exp_avg, self.exp_avg_sq = torch.zeros(total, **f32), torch.zeros(total, **f32)
         with torch.no_grad():
             for l, name, off, n, shape in offs:
                 p = getattr(l, name)
-                view = self.flat[off:off + n].view(shape)
-                view.copy_(p.data)
-                p.data = view
+                if process_group is None:
+                    view = self.flat[off:off + n].view(shape)
+                    view.copy_(p.data)
+                    p.data = view
                 p.grad = self.gflat[off:off + n].view(shape)
+        if process_group is not None:
+            # parameters move into the exchange's arena; the gradients stay in gflat, where lbbnn_vd_bwd writes them
+            self.opt = MultiTensorAdam([getattr(l, n) for l in self.layers for n in names], lr=self.lr, betas=betas,
+                                       eps=self.eps, weight_decay=self.wd)
+            self.opt.data_parallel(process_group)
+            self.dp_update = self.opt.dp["mode"]
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=dev)
         self.adam_coef = torch.zeros(2, **f32)
         B = self.B
@@ -228,11 +254,27 @@ class VDTrainer:
         self.graph = None
         if use_graph:
             self._capture()
+            if self.opt is not None:
+                self.opt.finish_capture()
 
     def _noise(self, i):
         if self.inject:
             return K.make_noise(self.buf[i]["zeta"])
-        return K.make_noise(None, self.seed, (0x5D << 56) | i, self.step_dev, len(self.layers))
+        return K.make_noise(None, self.seed + 0x9E3779B97F4A7C15 * self.rank, (0x5D << 56) | i, self.step_dev,
+                            len(self.layers))
+
+    def _train_state(self):
+        """What a step changes besides activations: restored after _capture's warm-up step, which must not count."""
+        if self.opt is None:
+            return self.flat, self.exp_avg, self.exp_avg_sq, self.step_dev
+        o = self.opt
+        return o.dp["arena"][:o.n_flat], o.exp_avg, o.exp_avg_sq, o.t_dev, self.step_dev
+
+    def owned_range(self, layer_index, name):
+        """Element range [lo, hi) of parameter `name` of layer `layer_index` whose AdamW moments THIS rank maintains: all of
+        it, except under the sharded data-parallel update (MultiTensorAdam.owned_range)."""
+        p = getattr(self.layers[layer_index], name)
+        return (0, p.numel()) if self.opt is None else self.opt.owned_range(p)
 
     def _enqueue(self):
         st = K.current_stream()
@@ -264,13 +306,18 @@ class VDTrainer:
                                      B, fi, fo, 0 if i == L - 1 else K.FLAG_RELU, P(l.theta.grad), P(d_alpha, True),
                                      P(dx, True), ws, wsn, st))
             n += 1 + lib.lbbnn_vd_gemm_launches(fi, fo, B) + (lib.lbbnn_vd_gemm_launches(B, fi, fo) if dx is not None else 0)
-            if self.train_alpha:
-                K.check(lib.lbbnn_vd_kl(P(l.alpha.data), fo, None, 0, P(l.alpha.grad), 1.0 / self.num_batches, st))
+            if self.train_alpha:      # the KL is replicated on every rank: its gradient is added once over the ranks
+                K.check(lib.lbbnn_vd_kl(P(l.alpha.data), fo, None, 0, P(l.alpha.grad), 1.0 / (self.num_batches * self.world),
+                                        st))
                 n += 1
-        K.check(lib.lbbnn_adamw_f32(P(self.flat), P(self.gflat), P(self.exp_avg), P(self.exp_avg_sq), self.n_flat, self.lr,
-                                    self.betas[0], self.betas[1], self.eps, self.wd, P(self.step_dev, torch.int64),
-                                    P(self.adam_coef), st))
-        n += 2
+        if self.opt is not None:
+            self.opt.step()       # pack, exchange, AdamW
+            n += 5 if self.dp_update == "sharded" else 4
+        else:
+            K.check(lib.lbbnn_adamw_f32(P(self.flat), P(self.gflat), P(self.exp_avg), P(self.exp_avg_sq), self.n_flat,
+                                        self.lr, self.betas[0], self.betas[1], self.eps, self.wd,
+                                        P(self.step_dev, torch.int64), P(self.adam_coef), st))
+            n += 2
         self.kernels_per_step = n
 
     _capture = LRTTrainer._capture
@@ -282,5 +329,7 @@ class VDTrainer:
     d2h_bytes_per_step = LRTTrainer.d2h_bytes_per_step
 
     def _stats_dict(self, st):
+        """Data parallel: `nll` and `loss` are THIS RANK's contribution (its rows, the replicated kl at 1 / world); their
+        sums over ranks are the single-GPU values of the concatenated minibatch.  `kl` is the replicated term."""
         nll, kl = float(st[0]), float(st[1])
-        return {"nll": nll, "kl": kl, "loss": nll + kl / self.num_batches}
+        return {"nll": nll, "kl": kl, "loss": nll + kl / (self.num_batches * self.world)}

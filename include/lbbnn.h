@@ -636,7 +636,10 @@ LBBNN_API int lbbnn_lrt_kl_finalize(const double* kl_part, int64_t n_part, const
  * for pa / pb, 1e-5 for the Gamma hyper-parameters, 0.1 for lambdal): table_dev = device array of n_entries records;
  * block b of the launch updates elements [(b - first_block) * 1024, +1024) of the tensor with the largest
  * first_block <= b, so first_block is the running sum of ceil(n / 1024) and total_blocks its final value.  Each entry's
- * learning rate is lr * lr_scale (its parameter group's lr relative to the call's). */
+ * learning rate is lr * lr_scale (its parameter group's lr relative to the call's).  decay = lr_group * weight_decay of the
+ * entry's group (computed by the caller: coef holds the bias-corrected step size, not the raw lr): non-zero makes the entry's
+ * update torch.optim.AdamW's (variational_dropout.py:110), param *= 1 - decay before the Adam step; 0 is torch.optim.Adam,
+ * bit for bit. */
 typedef struct lbbnn_adam_entry {
   float* param;
   const float* grad;
@@ -645,7 +648,7 @@ typedef struct lbbnn_adam_entry {
   int64_t n;
   int64_t first_block;
   float lr_scale;
-  float reserved;
+  float decay;
 } lbbnn_adam_entry;
 LBBNN_API int lbbnn_adam_multi_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, float lr,
                                    float beta1, float beta2, float eps, const int64_t* step_dev, float* coef_scratch,
@@ -655,15 +658,17 @@ LBBNN_API int lbbnn_adam_multi_f32(const lbbnn_adam_entry* table_dev, int n_entr
 LBBNN_API int lbbnn_adam_multi_step_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, float lr,
                                         float beta1, float beta2, float eps, int64_t* step_dev, float* coef_scratch,
                                         lbbnn_stream s);
-/* Data-parallel form of the table update above, for the training step of LBBNN-GP-MF-MNF.py:263-275 and
- * LBBNN-GP-MF.py:325-343 with the minibatch sharded over ranks: torch.optim.Adam of the SUM over ranks of the gradients.
+/* Data-parallel form of the table update above, for the training step of LBBNN-GP-MF-MNF.py:263-275,
+ * LBBNN-GP-MF.py:325-343 and variational_dropout.py:160-166 with the minibatch sharded over ranks: torch.optim.Adam (entries
+ * with decay != 0: torch.optim.AdamW) of the SUM over ranks of the gradients.
  * Every entry's param lies in one symmetric-memory arena [parameters | packed gradients] that is bound to an NVSwitch
  * multicast object (arena_mc is its multicast address), each tensor at a 16-byte aligned offset and padded with zeros to a
  * multiple of 4 floats; its packed gradient sits grad_offset floats (a multiple of 4) after it.
  *   pack:  param[grad_offset + i] = grad[i] for every entry -- this rank's gradients into its region of the arena.
  *   dp:    blocks [block_lo, block_hi) of the table (one rank's share, 1024 elements each; the ranks' shares cover every
  *          block once): in-switch sum over ranks of the packed gradient (multimem.ld_reduce), Adam on this rank's exp_avg /
- *          exp_avg_sq with lr * lr_scale, the new parameter stored to every rank's arena (multimem.st).  advance != 0:
+ *          exp_avg_sq with lr * lr_scale and the entry's decay, the new parameter stored to every rank's arena
+ *          (multimem.st).  advance != 0:
  *          *step_dev += 1 first, as lbbnn_adam_multi_step_f32; 0: as lbbnn_adam_multi_f32.
  * The caller orders the dp launch between two cross-rank barriers: every rank packed before, every store landed after. */
 LBBNN_API int lbbnn_adam_pack_f32(const lbbnn_adam_entry* table_dev, int n_entries, int64_t total_blocks, int64_t grad_offset,

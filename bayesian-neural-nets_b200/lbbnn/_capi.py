@@ -191,6 +191,9 @@ SIGNATURES = {
     "lbbnn_linear_f32_batched": (_INT, [_P, _I64, _P, _P, _INT, _I64, _I64, _I64, _INT, _P, _P]),
     "lbbnn_mc_accumulate_batched": (_INT, [_P, _INT, _I64, _I64, _P, _P, _P, _P]),
     "lbbnn_tf32_split": (_INT, [_P, _I64, _P, _P, _P]),
+    "lbbnn_lrt_mc_epilogue": (_INT, [_P, _I64, _P, _I64, _P, _P, _I64, _I64, _INT, C.POINTER(Noise), _U64, _INT, _P, _P,
+                                     _P, _P, _P, _P, _P]),
+    "lbbnn_tf32_split_rows": (_INT, [_P, _I64, _I64, _I64, _INT, _P, _P, _P, _P, _P, _P]),
     "lbbnn_mc_head_accumulate": (_INT, [_P, _I64, _P, _P, _INT, _I64, _I64, _I64, _P, _P, _P, _P]),
     "lbbnn_mc_prepare": (_INT, [C.POINTER(Layer), _P, _P, _P, _P]),
     "lbbnn_mc_sample_split": (_INT, [C.POINTER(Layer), _INT, _P, _U64, _U64, _U64, _INT, _P, _P, _P, _P]),

@@ -314,6 +314,27 @@ LBBNN_API int lbbnn_mc_accumulate_batched(const float* logits, int n_samples, in
  *                        All samples of a launch sharing one input (the first layer) = ONE problem with batches = 1 and
  *                        N = n_samples * out_features; its (batch, n_samples * out) output is the next layer's strided a. */
 LBBNN_API int lbbnn_tf32_split(const float* x, int64_t n, float* hi, float* lo, lbbnn_stream s);
+/* The LRT / MNF posterior-predictive loop (lbbnn.EnsemblePredictor) on the tensor cores (csrc/lrt_predict.cu): the LRT
+ * forward of n stacked samples is E = A_E M^T and S = A_S V^T (M, V from lbbnn_lrt_f32_prologue, split by lbbnn_tf32_split),
+ * each ONE lbbnn_tc_linear_tf32x3 call of n * batch rows with a zero bias; these two calls sit around them.
+ *   lrt_mc_epilogue   act[s] = [relu](E[s] + b_mu + sqrt(S[s] + sigma_b^2) eps_s) for s < n_samples, the expressions of the
+ *                     fp32 forward epilogue (LRT:172-175), sigma_b = log1p(exp bias_rho).  E[s] / S[s] (batch, out) start at
+ *                     E + s * e_sample_stride (0 = shared by all samples: layer 1 of an LRT network, MNF layer 1's S).  eps_s
+ *                     is injected ((n_samples, batch, out) in noise->eps) or drawn from stream_id + s * noise_group_stride
+ *                     with element index row * out + col -- the draws of lbbnn_lrt_f32_fwd_ex / lbbnn_lrt_sample_expand.
+ *                     Without FLAG_SAMPLE: act = [relu](E + b_mu) (LRT:177-180; S, bias_rho, noise unused).  Outputs, each
+ *                     (n_samples, batch, out), NULL = skip: act (fp32); m_hi / m_lo = split of act .* rowscale[s] (rowscale
+ *                     (n_samples, out) or NULL: the next MNF layer's z, MNF:197); v_hi / v_lo = split of act^2 (fp32 square).
+ *   tf32_split_rows   for s < n_samples: hi / lo of x[s] .* rowscale[s] and sq_hi / sq_lo of x[s]^2, where x[s] (rows, cols)
+ *                     starts at x + s * x_sample_stride (0 = one shared input); rowscale (n_samples, cols) or NULL; either
+ *                     output pair may be NULL.  Splits are lbbnn_tf32_split's (hi + lo == value, bit for bit). */
+LBBNN_API int lbbnn_lrt_mc_epilogue(const float* E, int64_t e_sample_stride, const float* S, int64_t s_sample_stride,
+                                    const float* bias_mu, const float* bias_rho, int64_t batch, int64_t out_features,
+                                    int n_samples, const lbbnn_noise* noise, uint64_t noise_group_stride, int flags,
+                                    float* act, const float* rowscale, float* m_hi, float* m_lo, float* v_hi, float* v_lo,
+                                    lbbnn_stream s);
+LBBNN_API int lbbnn_tf32_split_rows(const float* x, int64_t x_sample_stride, int64_t rows, int64_t cols, int n_samples,
+                                    const float* rowscale, float* hi, float* lo, float* sq_hi, float* sq_lo, lbbnn_stream s);
 /* Classifier head + accumulation in one launch: logits[s] = h[s] W[s]^T + bias[s] for the n_samples samples of a launch
  * (h: sample s at h + s * h_stride, (batch, in_features) row-major; W (n_samples, classes, in_features); classes <= 16,
  * in_features % 4 == 0, 16 (classes + 8) in_features <= 220 KB of shared memory), then exactly mc_accumulate_batched on them (same expressions, samples in order).  The logits

@@ -430,6 +430,12 @@ extern "C" int lbbnn_tc_linear_tf32x3(const float* a_hi, const float* a_lo, int6
   LBBNN_REQUIRE((out_hi == nullptr) == (out_lo == nullptr), "hi / lo outputs come in pairs");
   LBBNN_REQUIRE(M < (1LL << 31) && N < (1LL << 31) && K < (1LL << 31) && batches < 65536, "dims must fit int32");
   LBBNN_REQUIRE(K % 4 == 0, "contraction length must be a multiple of 4 (16-byte TMA pitch), got %lld", (long long)K);
+  // the epilogue stores float4 whenever both output pitches are multiples of 4 floats
+  LBBNN_REQUIRE(out_row_pitch % 4 != 0 || out_batch_stride % 4 != 0 ||
+                    ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(out_hi) |
+                      reinterpret_cast<uintptr_t>(out_lo)) & 15) == 0,
+                "outputs must be 16-byte aligned when their row pitch (%lld) and batch stride (%lld) are multiples of 4",
+                (long long)out_row_pitch, (long long)out_batch_stride);
   CUtensorMap mAh, mAl, mWh, mWl;
   if (int rc = make_map3(&mAh, a_hi, K, M, batches, a_row_pitch, a_batch_stride)) return rc;
   if (int rc = make_map3(&mAl, a_lo, K, M, batches, a_row_pitch, a_batch_stride)) return rc;

@@ -12,6 +12,8 @@
 // Operands are staged for either memory order (contraction index contiguous, or output index contiguous) so no transposed
 // copy of x, theta or the gradients ever exists.  Small-M problems split the contraction over gridDim.z; the partial sums
 // are added in a fixed order by the epilogue kernel, so results do not depend on the launch geometry of other calls.
+// lbbnn_vd_fwd_ex runs the forward over stacked MC samples for the predictive loop (lbbnn.vd.EnsemblePredictor): a native
+// noise stream per group of rows, or FLAG_MOMENTS (x theta and x^2 theta^2 without noise, once per test batch).
 #include "common.cuh"
 
 #include <algorithm>
@@ -26,10 +28,13 @@ enum { OP_FWD = 0, OP_AXPY = 1 };
 
 struct Epilogue {
   int op;
-  // OP_FWD: act = s1 + sqrt(s2 alpha[col]) zeta, ds = zeta / (2 sqrt(delta)), q = s2
+  // OP_FWD: act = s1 + sqrt(s2 alpha[col]) zeta, ds = zeta / (2 sqrt(delta)), q = s2;
+  //         moments: act = s1, ds = delta, q = s2 (no noise)
   const float* alpha;
   Noise noise;
-  int relu;
+  int64_t rows_per_group;  // native noise: row r of group g = r / rows_per_group draws element (r % rows_per_group) * N + col
+  uint64_t group_stride;   //   from stream noise.stream + g * group_stride
+  int relu, moments;
   float* act;
   float* ds;
   float* q;
@@ -43,8 +48,24 @@ __device__ __forceinline__ void apply_epilogue(const Epilogue& e, int64_t row, i
   const int64_t idx = row * N + col;
   if (e.op == OP_FWD) {
     const float delta = s2 * __ldg(e.alpha + col);
+    if (e.moments) {
+      e.act[idx] = s1;
+      if (e.ds) e.ds[idx] = delta;
+      if (e.q) e.q[idx] = s2;
+      return;
+    }
     const float sd = sqrtf(delta);
-    const float z = e.noise.ptr ? __ldg(e.noise.ptr + idx) : philox_normal1(e.noise.seed, e.noise.stream, (uint64_t)idx);
+    float z;
+    if (e.noise.ptr) {
+      z = __ldg(e.noise.ptr + idx);
+    } else {
+      const int64_t g = row / e.rows_per_group;
+      const uint64_t el = (uint64_t)((row - g * e.rows_per_group) * N + col);
+      float n4[4];      // philox_normal1, with the lane picked by selects (a dynamic index puts n4 on the stack here)
+      philox_normal4(e.noise.seed, e.noise.stream + (uint64_t)g * e.group_stride, el >> 2, n4);
+      const int lane = (int)(el & 3);
+      z = lane == 0 ? n4[0] : lane == 1 ? n4[1] : lane == 2 ? n4[2] : n4[3];
+    }
     float a = s1 + sd * z;
     if (e.relu) a = fmaxf(a, 0.f);
     e.act[idx] = a;
@@ -341,18 +362,32 @@ extern "C" int lbbnn_vd_gemm_launches(int64_t M, int64_t N, int64_t K) {
   return ceil_div(K, k_chunk) > 1 ? 2 : 1;
 }
 
-extern "C" int lbbnn_vd_fwd(const float* theta, const float* alpha, const float* x, int64_t batch, int64_t n, int64_t m,
-                            const lbbnn_noise* noise, int flags, float* act, float* ds_factor, float* q, void* workspace,
-                            size_t workspace_bytes, lbbnn_stream s) {
-  LBBNN_REQUIRE(theta && alpha && x && act && noise, "vd_fwd: null argument");
+extern "C" int lbbnn_vd_fwd_ex(const float* theta, const float* alpha, const float* x, int64_t batch, int64_t n, int64_t m,
+                               const lbbnn_noise* noise, int flags, float* act, float* ds_factor, float* q,
+                               int64_t rows_per_group, uint64_t noise_group_stride, void* workspace, size_t workspace_bytes,
+                               lbbnn_stream s) {
+  const bool moments = flags & LBBNN_FLAG_MOMENTS;
+  LBBNN_REQUIRE(theta && alpha && x && act && (noise || moments), "vd_fwd: null argument");
   LBBNN_REQUIRE(batch > 0 && n > 0 && m > 0, "vd_fwd: empty shape");
+  LBBNN_REQUIRE(rows_per_group > 0 && batch % rows_per_group == 0, "vd_fwd: batch %lld is not a multiple of rows_per_group %lld",
+                (long long)batch, (long long)rows_per_group);
   LBBNN_REQUIRE(on_device(theta) && on_device(x) && on_device(act), "vd_fwd: host pointer (there is no CPU fallback)");
   GemmArgs a{};
   a.A1 = x; a.B1 = theta;                 // A2 = x^2, B2 = theta^2 formed while staging
   a.M = batch; a.N = m; a.K = n; a.lda = n; a.ldb = m; a.a_kc = 1; a.b_kc = 0;
-  a.epi.op = OP_FWD; a.epi.alpha = alpha; a.epi.noise = make_noise(noise); a.epi.relu = (flags & LBBNN_FLAG_RELU) ? 1 : 0;
+  a.epi.op = OP_FWD; a.epi.alpha = alpha; a.epi.noise = make_noise(moments ? nullptr : noise);
+  a.epi.rows_per_group = rows_per_group; a.epi.group_stride = noise_group_stride;
+  a.epi.relu = (flags & LBBNN_FLAG_RELU) ? 1 : 0; a.epi.moments = moments ? 1 : 0;
   a.epi.act = act; a.epi.ds = ds_factor; a.epi.q = q;
   return launch_gemm(a, workspace, workspace_bytes, (cudaStream_t)s, "vd_fwd");
+}
+
+extern "C" int lbbnn_vd_fwd(const float* theta, const float* alpha, const float* x, int64_t batch, int64_t n, int64_t m,
+                            const lbbnn_noise* noise, int flags, float* act, float* ds_factor, float* q, void* workspace,
+                            size_t workspace_bytes, lbbnn_stream s) {
+  LBBNN_REQUIRE(noise, "vd_fwd: null argument");
+  return lbbnn_vd_fwd_ex(theta, alpha, x, batch, n, m, noise, flags & ~LBBNN_FLAG_MOMENTS, act, ds_factor, q, batch > 0 ? batch : 1,
+                         0, workspace, workspace_bytes, s);
 }
 
 extern "C" int lbbnn_vd_bwd(const float* theta, const float* alpha, const float* x, const float* act, const float* ds_factor,

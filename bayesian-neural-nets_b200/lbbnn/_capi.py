@@ -231,6 +231,10 @@ SIGNATURES = {
     "lbbnn_vd_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
     "lbbnn_vd_gemm_launches": (_INT, [_I64, _I64, _I64]),
     "lbbnn_vd_fwd": (_INT, [_P, _P, _P, _I64, _I64, _I64, C.POINTER(Noise), _INT, _P, _P, _P, _P, _SZ, _P]),
+    "lbbnn_vd_fwd_ex": (_INT, [_P, _P, _P, _I64, _I64, _I64, C.POINTER(Noise), _INT, _P, _P, _P, _I64, _U64, _P, _SZ, _P]),
+    "lbbnn_vd_tc_prepare": (_INT, [_P, _I64, _I64, _P, _P, _P, _P, _P]),
+    "lbbnn_vd_mc_epilogue": (_INT, [_P, _I64, _P, _I64, _P, _I64, _I64, _INT, C.POINTER(Noise), _U64, _INT, _P, _P, _P, _P,
+                                    _P, _P]),
     "lbbnn_vd_bwd": (_INT, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P, _SZ, _P]),
     "lbbnn_vd_kl": (_INT, [_P, _I64, _P, _INT, _P, _F, _P]),
 }

@@ -38,7 +38,59 @@ from .lrt import current_seed
 from .mf import shard_samples
 
 
-class EnsemblePredictor:
+class ShardedPredictor:
+    """What the batched posterior-predictive loops (EnsemblePredictor here, lbbnn.vd.EnsemblePredictor) share: the process
+    group (replica and seed checks at construction, contiguous sample shards, ONE all-reduce of the fp64 accumulators), the
+    sample count of result() and the 3xTF32 tensor-core GEMM of a layer.  Subclasses set device, seed, samples,
+    global_samples and zero_bias."""
+
+    def _join_group(self, process_group, params, what):
+        self.pg = process_group
+        if process_group is None:
+            return
+        import torch.distributed as dist
+        check_replicas(process_group, params, what)
+        seeds = [None] * dist.get_world_size(process_group)
+        dist.all_gather_object(seeds, self.seed, group=process_group)
+        if len(set(seeds)) != 1:
+            raise K.LbbnnError(f"{what}: ranks differ in the predictor seed: {seeds}")
+
+    def _reduce(self, sums):
+        """The fp64 accumulators `sums` over every rank: ONE all-reduce under a process group, this rank's own otherwise."""
+        if self.pg is None:
+            return tuple(sums)
+        both = torch.stack(tuple(sums))
+        torch.distributed.all_reduce(both, group=self.pg)
+        return tuple(both.unbind(0))
+
+    def _shard(self, samples):
+        """(first, count) of this rank's samples of a global run of `samples` (all of them without a process group)."""
+        if self.pg is None:
+            return 0, int(samples)
+        import torch.distributed as dist
+        return shard_samples(int(samples), dist.get_world_size(self.pg), dist.get_rank(self.pg))
+
+    def _total_samples(self, total_samples=None):
+        """The sample count result() divides by: `total_samples`, else the global count of the last run, else (under a
+        process group) the sum of the ranks' run() calls, else this process's."""
+        if total_samples is not None:
+            return int(total_samples)
+        if self.global_samples is not None:
+            return self.global_samples
+        if self.pg is not None:
+            n = torch.tensor([self.samples], dtype=torch.int64, device=self.device)
+            torch.distributed.all_reduce(n, group=self.pg)
+            return int(n.item())
+        return self.samples
+
+    def _gemm(self, a, w, rows, k, o, out, st):
+        """out (rows, o) = a w^T in 3xTF32, a and w as (hi, lo) pairs: ONE problem, the weights are shared by all samples."""
+        K.check(K.lib.lbbnn_tc_linear_tf32x3(K.ptr(a[0][:rows]), K.ptr(a[1][:rows]), k, 0, K.ptr(w[0]), K.ptr(w[1]),
+                                             K.ptr(self.zero_bias), 1, rows, o, k, 0, K.ptr(out[:rows * o]), None, None, o,
+                                             0, st))
+
+
+class EnsemblePredictor(ShardedPredictor):
     def __init__(self, net, batch, samples_per_launch=10, seed=None, gemm="auto", process_group=None):
         """gemm: "simt" = every layer on the fused fp32 CUDA-core kernels; "tc" = every layer with in_features % 4 == 0 on the
         tensor cores at fp32 accuracy (3xTF32, see the module docstring) except a <= 16-class head; "auto" = the tensor cores
@@ -56,14 +108,7 @@ class EnsemblePredictor:
         if dev.type != "cuda":
             raise K.LbbnnError("EnsemblePredictor needs the network on a CUDA device (no CPU fallback)")
         self.device = dev
-        self.pg = process_group
-        if process_group is not None:
-            import torch.distributed as dist
-            check_replicas(process_group, list(net.parameters()), "EnsemblePredictor")
-            seeds = [None] * dist.get_world_size(process_group)
-            dist.all_gather_object(seeds, self.seed, group=process_group)
-            if len(set(seeds)) != 1:
-                raise K.LbbnnError(f"EnsemblePredictor: ranks differ in the predictor seed: {seeds}")
+        self._join_group(process_group, list(net.parameters()), "EnsemblePredictor")
         f32 = dict(dtype=torch.float32, device=dev)
         self.sizes = sizes = [(l.in_features, l.out_features) for l in self.layers]
         L, B, SB, C = len(sizes), self.B, self.SB, sizes[-1][1]
@@ -156,12 +201,6 @@ class EnsemblePredictor:
         return self._z[li][s0 - self._z_start:s0 - self._z_start + n]
 
     # ---- tensor-core layers ------------------------------------------------------------------------------------------------
-    def _gemm(self, a, w, rows, k, o, out, st):
-        """out (rows, o) = a w^T in 3xTF32, a and w as (hi, lo) pairs: ONE problem, the weights are shared by all samples."""
-        K.check(K.lib.lbbnn_tc_linear_tf32x3(K.ptr(a[0][:rows]), K.ptr(a[1][:rows]), k, 0, K.ptr(w[0]), K.ptr(w[1]),
-                                             K.ptr(self.zero_bias), 1, rows, o, k, 0, K.ptr(out[:rows * o]), None, None, o,
-                                             0, st))
-
     def _prepare_weights(self, st, sample=True):
         """M (and, for the sampled forward, V) of every tensor-core layer as hi / lo, from the current parameters."""
         flag = K.FLAG_SAMPLE if sample else 0
@@ -344,33 +383,12 @@ class EnsemblePredictor:
     def _sums(self):
         """(sum_logp, sum_prob, first_logp, first_prob) over every rank: ONE all-reduce of the four fp64 accumulators under a
         process group, this rank's own otherwise."""
-        sums = (self.sum_logp, self.sum_prob, self.first_logp, self.first_prob)
-        if self.pg is None:
-            return sums
-        both = torch.stack(sums)
-        torch.distributed.all_reduce(both, group=self.pg)
-        return tuple(both.unbind(0))
-
-    def _shard(self, samples):
-        """(first, count) of this rank's samples of a global run of `samples` (all of them without a process group)."""
-        if self.pg is None:
-            return 0, int(samples)
-        import torch.distributed as dist
-        return shard_samples(int(samples), dist.get_world_size(self.pg), dist.get_rank(self.pg))
+        return self._reduce((self.sum_logp, self.sum_prob, self.first_logp, self.first_prob))
 
     def result(self, total_samples=None, first_k=10):
         """Statistics of the last run(); under a process group the accumulators are first summed over the ranks, and the
         default sample count is the global one (that of test_ensemble / outofsample, or the sum of the ranks' run() calls)."""
-        if total_samples is not None:
-            S = int(total_samples)
-        elif self.global_samples is not None:
-            S = self.global_samples
-        elif self.pg is not None:
-            n = torch.tensor([self.samples], dtype=torch.int64, device=self.device)
-            torch.distributed.all_reduce(n, group=self.pg)
-            S = int(n.item())
-        else:
-            S = self.samples
+        S = self._total_samples(total_samples)
         k = min(S, first_k)
         sum_logp, sum_prob, first_logp, _ = self._sums()
         probs = sum_prob / S

@@ -16,6 +16,7 @@ import torch.nn.functional as F
 from . import _capi as K
 from . import lrt as _lrt
 from .engine import LRTTrainer, MultiTensorAdam, check_replicas
+from .predict import ShardedPredictor
 
 _layer_ids = itertools.count(1)
 
@@ -162,13 +163,205 @@ def loss_fn(prediction, target, model, num_batches=600.0):
 
 
 def predict_ensemble(model, images, samples=10):
-    """The evaluation branch of run_epoch (VD:148-157): mean over `samples` stochastic forwards of the log-probabilities."""
+    """The evaluation branch of run_epoch (VD:148-157): mean over `samples` stochastic forwards of the log-probabilities.
+    EnsemblePredictor computes the same statistic with the samples batched on the device (and sharded over GPUs)."""
     with torch.no_grad():
         acc = None
         for _ in range(samples):
             out = model(images)
             acc = out if acc is None else acc + out
         return acc / samples
+
+
+class EnsemblePredictor(ShardedPredictor):
+    """predict_ensemble (the evaluation branch of run_epoch, VD:148-157) with the Monte-Carlo samples batched on the device:
+    the samples of a launch are stacked along the batch dimension and every layer runs ONCE per launch.
+
+      * layer 1 sees the same input in every sample: E1 = x theta and S1 = x^2 theta^2 are computed once per run()
+        (lbbnn_vd_fwd_ex with FLAG_MOMENTS, or two 3xTF32 GEMMs on the tensor cores) and every sample only adds its
+        sqrt(S1 alpha) zeta (lbbnn_vd_mc_epilogue with shared E and S);
+      * layers 2.. are ONE problem of samples_per_launch * batch rows: lbbnn_vd_fwd_ex with per-sample noise streams on the
+        CUDA cores, or E = A theta and S = A^2 theta^2 as two lbbnn_tc_linear_tf32x3 calls and lbbnn_vd_mc_epilogue on the
+        tensor cores (theta^T and (theta^2)^T split into hi / lo once per run() by lbbnn_vd_tc_prepare);
+      * log-softmax and the running sum stay on the device in fp64 (lbbnn_mc_accumulate_batched).
+
+    Sample g (global index) of layer l draws zeta from Philox stream (0x5E << 56) | (l + g * n_layers) of the predictor's
+    seed, so results do not depend on samples_per_launch, on sharding or on the GEMM path.  theta and alpha are read on
+    every run(); alpha may be the reference's buffer or a parameter (alpha_trainable=True).
+
+    gemm: "simt" = every layer on the CUDA cores; "tc" = every layer with in_features % 4 == 0 on the tensor cores at fp32
+    accuracy except a <= 16-class head; "auto" = the tensor cores for layers with in and out features both >= 1024 (the
+    784-1200-1200-1200-10 network: tc == [False, True, True, False]).
+    process_group: predict_ensemble shards its samples over the ranks and every rank gets the same result."""
+
+    STREAM_TAG = 0x5E << 56
+
+    def __init__(self, model, batch, samples_per_launch=10, seed=None, gemm="auto", process_group=None):
+        K.require_device()
+        if gemm not in ("auto", "simt", "tc"):
+            raise ValueError(f"gemm must be 'auto', 'simt' or 'tc', got {gemm!r}")
+        self.net, self.layers, self.B = model, list(model.layers), int(batch)
+        self.SB = max(1, int(samples_per_launch))
+        self.seed = _lrt.current_seed() if seed is None else int(seed)
+        dev = self.layers[0].theta.device
+        if dev.type != "cuda":
+            raise K.LbbnnError("vd.EnsemblePredictor needs the network on a CUDA device (no CPU fallback)")
+        self.device = dev
+        self._join_group(process_group, [getattr(l, n) for l in self.layers for n in ("theta", "alpha")],
+                         "vd.EnsemblePredictor")
+        self.sizes = sizes = [(l.n, l.m) for l in self.layers]
+        L, B, SB, C = len(sizes), self.B, self.SB, sizes[-1][1]
+        self.tc = [k % 4 == 0 and not (i == L - 1 and o <= 16) and (gemm == "tc" or (gemm == "auto" and k >= 1024 and o >= 1024))
+                   for i, (k, o) in enumerate(sizes)]
+        # layer 1 and the tensor-core layers end in lbbnn_vd_mc_epilogue, which writes the next tensor-core layer's operands
+        # directly; an fp32 output is kept where a CUDA-core layer or the head reads it, or a CUDA-core layer must split it
+        self._feeds_tc = [i + 1 < L and self.tc[i + 1] for i in range(L)]
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.x = torch.zeros(B, sizes[0][0], **f32)
+        self.E1, self.S1 = torch.zeros(B, sizes[0][1], **f32), torch.zeros(B, sizes[0][1], **f32)
+        self.h = [torch.zeros(SB * B, o, **f32) if not self._feeds_tc[i] or (i > 0 and not self.tc[i]) else None
+                  for i, (_, o) in enumerate(sizes)]
+        self.ws = torch.empty(max([workspace_bytes(B, *sizes[0])] + [workspace_bytes(SB * B, k, o) for k, o in sizes[1:]]),
+                              dtype=torch.uint8, device=dev)
+        f64 = dict(dtype=torch.float64, device=dev)
+        self.sum_logp, self.sum_prob = torch.zeros(B, C, **f64), torch.zeros(B, C, **f64)
+        self.kernels_per_launch = 0
+        self.samples, self.global_samples = 0, None
+        self.w, self.wsq, self.a, self.asq = {}, {}, {}, {}
+        if any(self.tc):
+            pair = lambda *shape: (torch.zeros(*shape, **f32), torch.zeros(*shape, **f32))      # noqa: E731
+            for i, (k, o) in enumerate(sizes):
+                if self.tc[i]:          # theta^T, (theta^2)^T (once per run()) and the inputs A, A^2 (the test batch for
+                    rows = B if i == 0 else SB * B      # layer 1, the stacked rows after it), all as hi / lo
+                    self.w[i], self.wsq[i] = pair(o, k), pair(o, k)
+                    self.a[i], self.asq[i] = pair(rows, k), pair(rows, k)
+            mo = max(o for (_, o), t in zip(sizes, self.tc) if t)
+            self.E, self.S = torch.zeros(SB * B * mo, **f32), torch.zeros(SB * B * mo, **f32)
+            self.zero_bias = torch.zeros(mo, **f32)
+
+    def _stream(self, layer, sample):
+        return self.STREAM_TAG | (layer + sample * len(self.layers))
+
+    def _noise_for(self, li, s0, off, n, zetas):
+        """(lbbnn_noise, group stride, keepalive) for the n samples with global indices s0 .. of layer li (injected zeta is
+        indexed by `off`: the position inside this run() call, or the global index under global_samples)."""
+        if zetas is not None:
+            z = zetas[li][off:off + n].reshape(n * self.B, self.sizes[li][1]).contiguous()
+            return K.make_noise(z), 0, z
+        return K.make_noise(None, self.seed, self._stream(li, s0)), len(self.layers), None
+
+    def _prepare(self, st):
+        """Per run(): theta^T, (theta^2)^T of the tensor-core layers as hi / lo, and layer 1's E1 = x theta, S1 = x^2 theta^2
+        for the test batch."""
+        for i in self.w:
+            k, o = self.sizes[i]
+            K.check(K.lib.lbbnn_vd_tc_prepare(K.ptr(self.layers[i].theta.data), k, o, K.ptr(self.w[i][0]), K.ptr(self.w[i][1]),
+                                              K.ptr(self.wsq[i][0]), K.ptr(self.wsq[i][1]), st))
+        l = self.layers[0]
+        k, o = self.sizes[0]
+        if self.tc[0]:
+            K.check(K.lib.lbbnn_tf32_split_rows(K.ptr(self.x), 0, self.B, k, 1, None, K.ptr(self.a[0][0]), K.ptr(self.a[0][1]),
+                                                K.ptr(self.asq[0][0]), K.ptr(self.asq[0][1]), st))
+            self._gemm(self.a[0], self.w[0], self.B, k, o, self.E1.view(-1), st)
+            self._gemm(self.asq[0], self.wsq[0], self.B, k, o, self.S1.view(-1), st)
+        else:
+            K.check(K.lib.lbbnn_vd_fwd_ex(K.ptr(l.theta.data), K.ptr(l.alpha.data), K.ptr(self.x), self.B, k, o, None,
+                                          K.FLAG_MOMENTS, K.ptr(self.E1), None, K.ptr(self.S1), self.B, 0, self.ws.data_ptr(),
+                                          self.ws.numel(), st))
+
+    def _layer(self, li, s0, off, n, zetas, h, st):
+        """Layer li for the n samples s0 .. of a launch (h: the stacked activations of layer li - 1); returns (its stacked
+        fp32 activations or None, the number of kernels it launched)."""
+        L, B = len(self.layers), self.B
+        l = self.layers[li]
+        k, o = self.sizes[li]
+        flags = 0 if li == L - 1 else K.FLAG_RELU
+        nz, gstride, keep = self._noise_for(li, s0, off, n, zetas)
+        out = None if self.h[li] is None else self.h[li][:n * B]
+        nxt = (self.a[li + 1], self.asq[li + 1]) if self._feeds_tc[li] else ((None, None), (None, None))
+        if li == 0 or self.tc[li]:
+            if li == 0:
+                E, es, S, ss, nk = self.E1, 0, self.S1, 0, 0
+            else:
+                self._gemm(self.a[li], self.w[li], n * B, k, o, self.E, st)
+                self._gemm(self.asq[li], self.wsq[li], n * B, k, o, self.S, st)
+                E, es, S, ss, nk = self.E, B * o, self.S, B * o, 2
+            K.check(K.lib.lbbnn_vd_mc_epilogue(K.ptr(E), es, K.ptr(S), ss, K.ptr(l.alpha.data), B, o, n, nz, gstride, flags,
+                                               K.ptr(None if self._feeds_tc[li] else out, True), K.ptr(nxt[0][0], True),
+                                               K.ptr(nxt[0][1], True), K.ptr(nxt[1][0], True), K.ptr(nxt[1][1], True), st))
+            return (None if self._feeds_tc[li] else out), nk + 1
+        K.check(K.lib.lbbnn_vd_fwd_ex(K.ptr(l.theta.data), K.ptr(l.alpha.data), K.ptr(h), n * B, k, o, nz, flags, K.ptr(out),
+                                      None, None, B, gstride, self.ws.data_ptr(), self.ws.numel(), st))
+        nk = K.lib.lbbnn_vd_gemm_launches(n * B, o, k)
+        if self._feeds_tc[li]:        # a CUDA-core layer feeding a tensor-core one
+            K.check(K.lib.lbbnn_tf32_split_rows(K.ptr(out), 0, n * B, o, 1, None, K.ptr(nxt[0][0]), K.ptr(nxt[0][1]),
+                                                K.ptr(nxt[1][0]), K.ptr(nxt[1][1]), st))
+            nk += 1
+        return out, nk
+
+    def _launch(self, s0, off, n, zetas):
+        st = K.current_stream()
+        nk, h = 0, None
+        for li in range(len(self.layers)):
+            h, k = self._layer(li, s0, off, n, zetas, h, st)
+            nk += k
+        K.check(K.lib.lbbnn_mc_accumulate_batched(K.ptr(h), n, self.B, self.sizes[-1][1], self.sum_logp.data_ptr(),
+                                                  self.sum_prob.data_ptr(), None, st))
+        self.kernels_per_launch = nk + 1
+
+    def _check_inputs(self, x, zetas, end):
+        B, n0 = self.B, self.sizes[0][0]
+        if not torch.is_tensor(x) or not x.is_cuda:
+            raise K.LbbnnError("vd.EnsemblePredictor takes CUDA inputs only (no CPU fallback)")
+        if x.numel() != B * n0 or x.shape[0] != B:
+            raise K.LbbnnError(f"input must be ({B}, {n0}) (or reshape to it), got {tuple(x.shape)}")
+        if zetas is not None:
+            if len(zetas) != len(self.layers):
+                raise K.LbbnnError(f"zetas: one tensor per layer ({len(self.layers)}), got {len(zetas)}")
+            for z, (_, o) in zip(zetas, self.sizes):
+                if z.dim() != 3 or tuple(z.shape[1:]) != (B, o) or z.shape[0] < end:
+                    raise K.LbbnnError(f"zetas: expected (>= {end}, {B}, {o}) per layer, got {tuple(z.shape)}")
+
+    @torch.no_grad()
+    def run(self, x, samples, first_sample=0, zetas=None, global_samples=None):
+        """Accumulate `samples` stochastic forwards (global sample indices first_sample ..) of the input batch x into the
+        fp64 sum_logp.  zetas: optional injected N(0,1) noise, one (S, batch, out) tensor per layer.  global_samples: this
+        call runs part of a run over samples 0 .. global_samples (one rank's shard), and zetas are indexed by global sample;
+        without it they are indexed from first_sample."""
+        st = K.current_stream()
+        first, count = int(first_sample), int(samples)
+        base = first if global_samples is None else 0
+        if global_samples is not None and first + count > int(global_samples):
+            raise ValueError(f"samples {first} .. {first + count} lie outside the global run of {global_samples}")
+        self._check_inputs(x, zetas, first + count - base)
+        self.x.copy_(x.reshape(self.x.shape))
+        self.sum_logp.zero_()
+        self.sum_prob.zero_()
+        self._prepare(st)
+        s, end = first, first + count
+        while s < end:
+            n = min(self.SB, end - s)
+            self._launch(s, s - base, n, zetas)
+            s += n
+        self.samples = count
+        self.global_samples = None if global_samples is None else int(global_samples)
+
+    def result(self, total_samples=None):
+        """mean_logp (fp64, (batch, classes)) and its argmax over the samples of the last run(); under a process group the
+        sums are first added over the ranks and the default sample count is the global one."""
+        S = self._total_samples(total_samples)
+        (sum_logp,) = self._reduce((self.sum_logp,))
+        mean = sum_logp / S
+        return {"mean_logp": mean, "pred": mean.argmax(1)}
+
+    @torch.no_grad()
+    def predict_ensemble(self, images, samples, zetas=None):
+        """What predict_ensemble(model, images, samples) returns: the fp32 mean over `samples` stochastic forwards of the
+        log-probabilities.  Under a process group each rank runs its share of the samples and every rank returns the same
+        value; injected zetas are indexed by global sample."""
+        first, count = self._shard(samples)
+        self.run(images, count, first_sample=first, zetas=zetas, global_samples=None if self.pg is None else samples)
+        return self.result(samples)["mean_logp"].float()
 
 
 class VDTrainer:

@@ -722,6 +722,34 @@ LBBNN_API int lbbnn_vd_gemm_launches(int64_t M, int64_t N, int64_t K);
 LBBNN_API int lbbnn_vd_fwd(const float* theta, const float* alpha, const float* x, int64_t batch, int64_t n, int64_t m,
                            const lbbnn_noise* noise, int flags, float* act, float* ds_factor, float* q, void* workspace,
                            size_t workspace_bytes, lbbnn_stream s);
+/* The same forward for the batched posterior-predictive loop (lbbnn.vd.EnsemblePredictor), where `batch` stacks
+ * rows_per_group input rows for each of several MC samples (batch % rows_per_group == 0):
+ *   native noise per group: rows of group g draw from stream_id + g * noise_group_stride with element index
+ *     (row - g * rows_per_group) * m + col, i.e. what a rows_per_group-row call on that stream draws (injected noise is
+ *     indexed like act);
+ *   FLAG_MOMENTS: no noise (may be NULL); act <- x theta, ds_factor <- delta = (x^2 theta^2) alpha, q <- x^2 theta^2 --
+ *     what layer 1 computes once per test batch when all samples share the input, expanded by lbbnn_vd_mc_epilogue.
+ * lbbnn_vd_fwd is this call with rows_per_group = batch. */
+LBBNN_API int lbbnn_vd_fwd_ex(const float* theta, const float* alpha, const float* x, int64_t batch, int64_t n, int64_t m,
+                              const lbbnn_noise* noise, int flags, float* act, float* ds_factor, float* q,
+                              int64_t rows_per_group, uint64_t noise_group_stride, void* workspace, size_t workspace_bytes,
+                              lbbnn_stream s);
+/* The tensor-core side of that loop (csrc/vd_predict.cu): the forward of n stacked samples is E = A theta and
+ * S = A^2 theta^2, each ONE lbbnn_tc_linear_tf32x3 call of n * batch rows with a zero bias, around which sit
+ *   vd_tc_prepare    t_hi / t_lo = split of theta^T and sq_hi / sq_lo = split of (theta .* theta)^T (fp32 square), all
+ *                    (m, n): the K-major weight operands of lbbnn_tc_linear_tf32x3, from theta (n, m), one tiled transpose;
+ *   vd_mc_epilogue   act[s] = [relu](E[s] + sqrtf(S[s] alpha[col]) zeta_s) for s < n_samples, the expressions of the vd_fwd
+ *                    epilogue.  E[s] / S[s] (batch, out) start at E + s * e_sample_stride (0 = shared by all samples: layer 1,
+ *                    from FLAG_MOMENTS or from its two GEMMs over the test batch).  zeta_s is injected ((n_samples, batch, out)
+ *                    in noise->eps) or drawn from stream_id + s * noise_group_stride with element index row * out + col --
+ *                    the draws of lbbnn_vd_fwd_ex.  Outputs, each (n_samples, batch, out), NULL = skip: act (fp32);
+ *                    a_hi / a_lo = split of act; sq_hi / sq_lo = split of act^2 (fp32 square). */
+LBBNN_API int lbbnn_vd_tc_prepare(const float* theta, int64_t n, int64_t m, float* t_hi, float* t_lo, float* sq_hi,
+                                  float* sq_lo, lbbnn_stream s);
+LBBNN_API int lbbnn_vd_mc_epilogue(const float* E, int64_t e_sample_stride, const float* S, int64_t s_sample_stride,
+                                   const float* alpha, int64_t batch, int64_t out_features, int n_samples,
+                                   const lbbnn_noise* noise, uint64_t noise_group_stride, int flags, float* act, float* a_hi,
+                                   float* a_lo, float* sq_hi, float* sq_lo, lbbnn_stream s);
 LBBNN_API int lbbnn_vd_bwd(const float* theta, const float* alpha, const float* x, const float* act, const float* ds_factor,
                            const float* q, const float* gact, int64_t batch, int64_t n, int64_t m, int flags,
                            float* d_theta, float* d_alpha, float* dx, void* workspace, size_t workspace_bytes,

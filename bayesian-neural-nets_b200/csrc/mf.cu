@@ -13,7 +13,7 @@
 //                   s4 = sum g log(alpha+1e-8) + (1-g) log(1-alpha+1e-8)      (Bernoulli.log_prob, MF:122-128)
 //   mf_sample_bwd autograd of the above: (dL/dw, dL/ds0..4) -> dmu, drho, dlambda, dgamma, dpb
 // All vectorised (float4) and coalesced; reductions are two-stage with a fixed order (deterministic).
-#include "common.cuh"
+#include "mf_math.cuh"
 
 #include <cstdlib>
 
@@ -22,7 +22,6 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kLpWidthDefault = 2;   // see lp_width(): same-box A/B 0.2734 (4) / 0.2641 (2) / 0.2644 (1) ms per MF step
-constexpr float kLogSqrt2Pi = 0.91893853320467274178f;
 
 __device__ __forceinline__ void ldq(const float* __restrict__ p, int64_t e0, int64_t n, bool vec, float out[4]) {
   if (vec && e0 + 3 < n) {
@@ -90,18 +89,6 @@ __device__ __forceinline__ void pickw(const float (&g4)[4], int sub, float (&out
   }
 }
 
-// digamma for x > 0: recurrence up to x >= 6, then the asymptotic series
-__device__ __forceinline__ float digammaf(float x) {
-  float r = 0.f;
-  while (x < 6.0f) { r -= 1.0f / x; x += 1.0f; }
-  const float f = 1.0f / (x * x);
-  return r + logf(x) - 0.5f / x - f * (1.0f / 12.0f - f * (1.0f / 120.0f - f * (1.0f / 252.0f - f * (1.0f / 240.0f - f / 132.0f))));
-}
-
-__device__ __forceinline__ float clampf(float v, float lo, float hi) { return fminf(fmaxf(v, lo), hi); }
-constexpr float kEps = 1.1920928955078125e-07f;   // torch.finfo(float32).eps
-constexpr float kTiny = 1.1754943508222875e-38f;  // torch.finfo(float32).tiny
-
 // ---- gamma.rsample ----------------------------------------------------------------------------------
 struct GammaArgs {
   const float *lam, *alpha_in;  // one of them: alpha = sigmoid(lam) or the given tensor
@@ -127,13 +114,7 @@ __global__ void __launch_bounds__(kThreads) mf_gamma_kernel(const GammaArgs a) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const float al = a.lam ? alpha_of(s[j]) : s[j];
-      if (a.exact) {
-        g[j] = u[j] < al ? 1.0f : 0.0f;
-      } else {  // torch RelaxedBernoulli.rsample: clamp_probs, logistic noise, /T, clipped sigmoid
-        const float p = clampf(al, kEps, 1.0f - kEps), uu = clampf(u[j], kEps, 1.0f - kEps);
-        const float logits = (logf(uu) - log1pf(-uu) + logf(p) - log1pf(-p)) * a.inv_t;
-        g[j] = clampf(1.0f / (1.0f + expf(-logits)), kTiny, 1.0f - kEps);
-      }
+      g[j] = a.exact ? (u[j] < al ? 1.0f : 0.0f) : relaxed_bernoulli(al, u[j], a.inv_t);
     }
     stq(a.gamma, e0, a.n, vec, g);
   }
@@ -145,13 +126,7 @@ __global__ void __launch_bounds__(kThreads) mf_gamma_bwd_kernel(const float* __r
                                                                 int64_t n, float inv_t, float* __restrict__ dout) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const float al = lam ? alpha_of(lam[i]) : alpha_in[i];
-    const float g = gamma[i];
-    float d = 0.f;
-    if (g > kTiny && g < 1.0f - kEps && al > kEps && al < 1.0f - kEps) {
-      d = dgamma[i] * g * (1.0f - g) * inv_t * (1.0f / al + 1.0f / (1.0f - al));
-      if (lam) d *= al * (1.0f - al);
-    }
-    dout[i] = d;
+    dout[i] = relaxed_bernoulli_bwd(dgamma[i], gamma[i], al, inv_t, lam != nullptr);
   }
 }
 
@@ -265,16 +240,7 @@ __global__ void __launch_bounds__(kThreads) mf_sample_kernel(const SampleArgs a)
       if (a.want_lp) {
         if (a.mode != LBBNN_MF_SAMPLE) sg = sigma_of(rho[j]);
         const float al = alpha_of(lam[j]);
-        const float wl = a.lp_on_ws ? ws : w[j];
-        const float gr = rintf(g);
-        const float g_wp = a.exact_wp ? gr : g, g_gp = a.exact_gp ? gr : g, g_b = a.exact_b ? gr : g;
-        s[0] += g_wp;
-        s[1] += wl * wl;
-        s[2] += lgammaf(1.0f + pb - g_gp) - lgammaf(2.0f - g_gp);
-        const float dlt = wl - mu[j];
-        const float logn = -kLogSqrt2Pi - logf(sg) - (dlt * dlt) / (2.0f * sg * sg);
-        s[3] += logf(g * expf(logn) + (1.0f - g) + 1e-8f);
-        s[4] += g_b * logf(al + 1e-8f) + (1.0f - g_b) * logf(1.0f - al + 1e-8f);
+        mf_lp_terms(g, a.lp_on_ws ? ws : w[j], mu[j], sg, al, pb, a.exact_b, a.exact_wp, a.exact_gp, s);
       }
     }
     stw<W>(a.w, e0, a.n, vec, w);
@@ -357,29 +323,13 @@ __global__ void __launch_bounds__(kThreads) mf_sample_bwd_kernel(const SampleBwd
     for (int j = 0; j < W; ++j) {
       gm[j] = gr[j] = gl[j] = gg[j] = 0.f;
       if (e0 + j >= a.n) continue;
-      const float sg = sigma_of(rho[j]), al = alpha_of(lam[j]), g = ga[j];
-      const float ws = fmaf(sg, ep[j], mu[j]), w = g * ws, wl = a.lp_on_ws ? ws : w;
-      const float grd = rintf(g);
-      const float g_gp = a.exact_gp ? grd : g, g_b = a.exact_b ? grd : g;
-      const float dlt = wl - mu[j], inv_s2 = 1.0f / (sg * sg);
-      const float logn = -kLogSqrt2Pi - logf(sg) - (dlt * dlt) * 0.5f * inv_s2;
-      const float p = expf(logn), D = g * p + (1.0f - g) + 1e-8f, r = g * p / D;
-      const float dwl = c[1] * 2.0f * wl - c[3] * r * dlt * inv_s2;          // direct dL/d(wl)
-      const float dmu_dir = c[3] * r * dlt * inv_s2;
-      const float dsg_dir = c[3] * r * (dlt * dlt * inv_s2 / sg - 1.0f / sg);
-      const float psi = digammaf(1.0f + pb - g_gp);
-      psisum += psi;
-      float dg_dir = c[3] * (p - 1.0f) / D;
-      if (!a.exact_wp) dg_dir += c[0];
-      if (!a.exact_gp) dg_dir += c[2] * (digammaf(2.0f - g_gp) - psi);
-      if (!a.exact_b) dg_dir += c[4] * (logf(al + 1e-8f) - logf(1.0f - al + 1e-8f));
-      const float dal = c[4] * (g_b / (al + 1e-8f) - (1.0f - g_b) / (1.0f - al + 1e-8f));
-      const float dw_tot = dw[j] + (a.lp_on_ws ? 0.f : dwl);
-      const float dws = g * dw_tot + (a.lp_on_ws ? dwl : 0.f);
-      gm[j] = dws + dmu_dir;
-      gr[j] = (ep[j] * dws + dsg_dir) * dsigma_drho(rho[j]);
-      gl[j] = dal * al * (1.0f - al);
-      gg[j] = ws * dw_tot + dg_dir;
+      const MfElemGrad e = mf_lp_terms_bwd(c, mu[j], rho[j], lam[j], ga[j], ep[j], dw[j], pb, a.lp_on_ws, a.exact_b,
+                                           a.exact_wp, a.exact_gp);
+      psisum += e.psi;
+      gm[j] = e.dmu;
+      gr[j] = e.drho;
+      gl[j] = e.dlam;
+      gg[j] = e.dgamma;
     }
     stw<W>(a.dmu, e0, a.n, vec, gm);
     stw<W>(a.drho, e0, a.n, vec, gr);
@@ -478,20 +428,12 @@ __global__ void __launch_bounds__(kThreads) mf_prior_fwd_kernel(PriorArgs a) {
     const float bias = a.sample ? mu + sb * e : mu;
     a.bias[i] = bias;
     a.eps_out[i] = e;
-    const float ba = __ldg(a.ba + i), bb = __ldg(a.bb + i), tb = __ldg(a.tau_b + i);
-    const float cb = ba * logf(bb) + (ba - 0.5f) * tb - bb * tb - lgammaf(ba) - kLogSqrt2Pi;
-    gb += cb - tb * bias * bias + 1e-8f;
-    const float d = bias - mu;
-    lq += -kLogSqrt2Pi - logf(sb) - (d * d) / (2.0f * sb * sb);
+    mf_bias_lp_terms(bias, mu, sb, __ldg(a.ba + i), __ldg(a.bb + i), __ldg(a.tau_b + i), gb, lq);
   }
   gb = block_sum(gb, red);
   lq = block_sum(lq, red);
   if (threadIdx.x == 0) {
-    const float av = a.a[0], bv = a.b[0], tw = a.tau_w[0], pa = a.pa[0], pb = a.pb[0];
-    const float cw = av * logf(bv) + (av - 0.5f) * tw - bv * tw - lgammaf(av) - kLogSqrt2Pi;
-    const float ggw = a.s[0] * cw - tw * a.s[1] + (a.n - a.s[0]) + a.n * 1e-8f;
-    const float bbin = a.s[2] + a.n * (lgammaf(pa + pb) - lgammaf(1.0f + pa + pb) - lgammaf(pa) - lgammaf(pb));
-    a.lp[0] = ggw + gb + bbin;
+    a.lp[0] = mf_log_prior(a.s, gb, a.a[0], a.b[0], a.tau_w[0], a.pa[0], a.pb[0], a.n);
     a.lp[1] = a.s[3] + a.s[4] + lq;
   }
 }
@@ -511,45 +453,19 @@ struct PriorBwdArgs {
 __global__ void __launch_bounds__(kThreads) mf_prior_bwd_kernel(const PriorBwdArgs a) {
   const float gp = a.g_lp ? __ldg(a.g_lp) : 0.f, gq = a.g_lq ? __ldg(a.g_lq) : 0.f;
   for (int i = threadIdx.x; i < a.out; i += kThreads) {
-    const float mu = __ldg(a.bias_mu + i), rho = __ldg(a.bias_rho + i), sb = sigma_of(rho);
-    const float bias = __ldg(a.bias + i), e = __ldg(a.eps + i), d = bias - mu;
-    const float ba = __ldg(a.ba + i), bb = __ldg(a.bb + i), tb = __ldg(a.tau_b + i);
-    const float dtb = gp * ((ba - 0.5f) - bb - bias * bias);
-    float dba = gp * (logf(bb) + tb - digammaf(ba)), dbb = gp * (ba / bb - tb);
-    if (a.tb_da) {
-      dba = fmaf(dtb, __ldg(a.tb_da + i), dba);
-      dbb = fmaf(dtb, __ldg(a.tb_db + i), dbb);
-    }
-    a.d_ba[i] = dba;
-    a.d_bb[i] = dbb;
-    a.d_tau_b[i] = dtb;
-    const float inv2 = 1.0f / (sb * sb);
-    const float G = (a.g_bias ? __ldg(a.g_bias + i) : 0.f) + gp * (-2.0f * tb * bias) + gq * (-d * inv2);   // d loss / d bias
-    a.d_bias_mu[i] = G + gq * (d * inv2);
-    const float dsb = (a.sample ? G * e : 0.f) + gq * (-1.0f / sb + d * d * inv2 / sb);
-    a.d_bias_rho[i] = dsb * dsigma_drho(rho);
+    const MfBiasGrad g = mf_bias_lp_terms_bwd(gp, gq, a.g_bias ? __ldg(a.g_bias + i) : 0.f, __ldg(a.bias_mu + i),
+                                              __ldg(a.bias_rho + i), __ldg(a.bias + i), __ldg(a.eps + i), __ldg(a.ba + i),
+                                              __ldg(a.bb + i), __ldg(a.tau_b + i), a.sample, a.tb_da != nullptr,
+                                              a.tb_da ? __ldg(a.tb_da + i) : 0.f, a.tb_da ? __ldg(a.tb_db + i) : 0.f);
+    a.d_ba[i] = g.dba;
+    a.d_bb[i] = g.dbb;
+    a.d_tau_b[i] = g.dtb;
+    a.d_bias_mu[i] = g.dmu;
+    a.d_bias_rho[i] = g.drho;
   }
   if (threadIdx.x == 0) {
-    const float av = a.a[0], bv = a.b[0], tw = a.tau_w[0], pa = a.pa[0], pb = a.pb[0];
-    const float cw = av * logf(bv) + (av - 0.5f) * tw - bv * tw - lgammaf(av) - kLogSqrt2Pi;
-    const float s0 = a.s[0], s1 = a.s[1];
-    a.d_scalar[0] = gp * (cw - 1.0f);
-    a.d_scalar[1] = gp * (-tw);
-    a.d_scalar[2] = gp;
-    a.d_scalar[3] = gq;
-    a.d_scalar[4] = gq;
-    const float dtw = gp * (s0 * ((av - 0.5f) - bv) - s1);
-    float da = gp * s0 * (logf(bv) + tw - digammaf(av)), db = gp * s0 * (av / bv - tw);
-    if (a.tw_da) {
-      da = fmaf(dtw, a.tw_da[0], da);
-      db = fmaf(dtw, a.tw_db[0], db);
-    }
-    a.d_scalar[5] = da;
-    a.d_scalar[6] = db;
-    a.d_scalar[7] = dtw;
-    const float psi_s = digammaf(pa + pb) - digammaf(1.0f + pa + pb);
-    a.d_scalar[8] = gp * a.n * (psi_s - digammaf(pa));
-    a.d_scalar[9] = gp * a.n * (psi_s - digammaf(pb));
+    mf_log_prior_bwd(gp, gq, a.s[0], a.s[1], a.a[0], a.b[0], a.tau_w[0], a.pa[0], a.pb[0], a.n, a.tw_da != nullptr,
+                     a.tw_da ? a.tw_da[0] : 0.f, a.tw_da ? a.tw_db[0] : 0.f, a.d_scalar);
   }
 }
 

@@ -120,6 +120,17 @@ class Step(C.Structure):
                 ("kl_scale", C.c_float), ("stats", C.c_void_p), ("dp", C.POINTER(StepDp))]
 
 
+MFSIM_MAX_IN = 32
+
+
+class MfSim(C.Structure):
+    _fields_ = [("replicas", C.c_int64), ("in_features", C.c_int64), ("rows", C.c_int64), ("batch", C.c_int64),
+                ("params", C.c_void_p), ("param_stride", C.c_int64), ("x", C.c_void_p), ("x_stride", C.c_int64),
+                ("y", C.c_void_p), ("y_stride", C.c_int64), ("lr", C.c_float * 11), ("num_batches", C.c_float),
+                ("temperature", C.c_float), ("flags", C.c_int), ("seed", C.c_uint64), ("step", C.c_void_p)] + [
+        (n, C.c_void_p) for n in ("eps_w", "eps_b", "g0_w", "g0_b", "u", "gamma", "stats", "grads")]
+
+
 _P, _I64, _U64, _INT, _F, _SZ = C.c_void_p, C.c_int64, C.c_uint64, C.c_int, C.c_float, C.c_size_t
 
 # name -> (restype, argtypes); kept in one table so tests can check every header symbol is bound
@@ -237,6 +248,8 @@ SIGNATURES = {
                                     _P, _P]),
     "lbbnn_vd_bwd": (_INT, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _INT, _P, _P, _P, _P, _SZ, _P]),
     "lbbnn_vd_kl": (_INT, [_P, _I64, _P, _INT, _P, _F, _P]),
+    "lbbnn_mfsim_train_f32": (_INT, [C.POINTER(MfSim), _INT, _P]),
+    "lbbnn_philox_std_gamma": (_INT, [_F, _I64, _U64, _U64, _P, _P]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():
@@ -382,6 +395,14 @@ def philox_normal(shape, seed, stream_id, device="cuda"):
     require_device()
     out = torch.empty(shape, dtype=torch.float32, device=device)
     check(lib.lbbnn_philox_normal(ptr(out), out.numel(), seed, stream_id, current_stream()))
+    return out
+
+
+def philox_std_gamma(a, n, seed, stream_id, device="cuda"):
+    """n standard-Gamma(a) draws of stream (seed, stream_id) -- the sampler of the simulation-study kernel."""
+    require_device()
+    out = torch.empty(n, dtype=torch.float32, device=device)
+    check(lib.lbbnn_philox_std_gamma(float(a), n, seed & (2 ** 64 - 1), stream_id & (2 ** 64 - 1), ptr(out), current_stream()))
     return out
 
 

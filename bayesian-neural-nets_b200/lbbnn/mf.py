@@ -7,6 +7,7 @@ The O(1)/O(out) hyper-prior glue (Gamma(a,b).rsample(), the (a,b,tau) and (pa,pb
 terms) stays in torch on the device, exactly where the reference has it, so autograd reaches
 weight_a/weight_b/bias_a/bias_b/pa/pb unchanged.
 """
+import ctypes as C
 import math
 import os
 
@@ -572,6 +573,152 @@ class SimStudyNetwork(nn.Module):
         log_prior, log_q, nll = torch.stack(lps).mean(), torch.stack(lqs).mean(), torch.stack(nlls).mean()
         loss = nll + (log_q - log_prior) / self.num_batches
         return loss, log_prior, log_q, nll, torch.stack(outs).mean(0)
+
+
+# the 11 tensors of a sim-study layer in the packed order of lbbnn_mfsim (include/lbbnn.h) and the study's SGD learning
+# rates (MFsim:359-374)
+SIM_PARAM_NAMES = ("weight_mu", "weight_rho", "lambdal", "bias_mu", "bias_rho", "weight_a", "weight_b", "bias_a", "bias_b",
+                   "pa", "pb")
+SIM_STUDY_LRS = {"weight_mu": 1e-4, "weight_rho": 1e-4, "lambdal": 1e-3, "bias_mu": 1e-4, "bias_rho": 1e-4, "weight_a": 1e-3,
+                 "weight_b": 1e-3, "bias_a": 1e-3, "bias_b": 1e-3, "pa": 1e-3, "pb": 1e-3}
+_SIM_NOISE = ("eps_w", "eps_b", "g0_w", "g0_b")
+
+
+class SimStudyEnsemble:
+    """Every repetition of the simulation study (MFsim:344-429) trained in ONE kernel launch (csrc/mf_sim.cu): R
+    SimStudyNetwork replicas, each running sample_elbo + backward + per-tensor SGD for whole epochs over minibatches of
+    `batch_size` consecutive rows of X.
+
+    The replicas' parameters live in one packed (R, P) device buffer; every module's nn.Parameters are re-pointed at views of
+    it (and, with materialize_grads, their .grad at the last step's gradients), so state_dict() and eager sample_elbo keep
+    working on each replica.  X is (n, in) shared by every replica or (R, n, in); y the {0, 1} targets (n,) or (R, n).
+    lrs: None = the study's rates (SIM_STUDY_LRS); a dict overrides per tensor name.  Native noise is Philox keyed by
+    (seed, replica, the replica's step, kind of draw).  The `.exact` flags of gamma / weight_prior / gamma_prior are read from
+    the modules at every run()."""
+
+    def __init__(self, nets, X, y, batch_size=400, lrs=None, seed=0, materialize_grads=True):
+        nets = list(nets)
+        if not nets:
+            raise K.LbbnnError("SimStudyEnsemble needs at least one network")
+        layers = [n.l1 for n in nets]
+        in_f = layers[0].in_features
+        for n, l in zip(nets, layers):
+            if (l.in_features, l.out_features) != (in_f, 1):
+                raise K.LbbnnError(f"every replica must be an {in_f} -> 1 SimStudyNetwork, got {l.in_features} -> {l.out_features}")
+            if not l.logprob_on_ws:
+                raise K.LbbnnError("the replicas must evaluate their log-probabilities at the unmasked ws (SimStudyNetwork)")
+            if float(n.num_batches) != float(nets[0].num_batches) or float(l.gamma.temperature) != float(layers[0].gamma.temperature):
+                raise K.LbbnnError("the replicas' num_batches and gamma temperature must agree")
+        if in_f > K.MFSIM_MAX_IN:
+            raise K.LbbnnError(f"in_features = {in_f} is above the kernel's limit of {K.MFSIM_MAX_IN}")
+        R = len(nets)
+        if X.dim() == 2:
+            n = X.shape[0]
+        elif X.dim() == 3 and X.shape[0] == R:
+            n = X.shape[1]
+        else:
+            raise K.LbbnnError(f"X must be (n, {in_f}) or ({R}, n, {in_f}), got {tuple(X.shape)}")
+        if X.shape[-1] != in_f:
+            raise K.LbbnnError(f"X has {X.shape[-1]} features, the networks {in_f}")
+        if tuple(y.shape) not in ((n,), (R, n)):
+            raise K.LbbnnError(f"y must be ({n},) or ({R}, {n}), got {tuple(y.shape)}")
+        B = int(batch_size)
+        if B < 1 or n % B:
+            raise K.LbbnnError(f"the {n} rows are not a whole number of minibatches of {B}")
+        rates = dict(SIM_STUDY_LRS)
+        if lrs is not None:
+            unknown = set(lrs) - set(SIM_PARAM_NAMES)
+            if unknown:
+                raise K.LbbnnError(f"unknown parameter names in lrs: {sorted(unknown)}")
+            rates.update(lrs)
+        self._flags_of(layers)
+        params = [getattr(l, name) for l in layers for name in SIM_PARAM_NAMES]
+        if any(not p.is_cuda for p in params) or not X.is_cuda or not y.is_cuda:
+            raise K.LbbnnError("SimStudyEnsemble takes CUDA networks and data (no CPU fallback)")
+        dev = params[0].device
+        if any(p.device != dev for p in params) or X.device != dev or y.device != dev:
+            raise K.LbbnnError("networks and data must live on one device")
+        K.require_device()
+        self.nets, self.layers, self.R, self.in_features, self.rows, self.batch = nets, layers, R, in_f, n, B
+        self.num_batches, self.temperature = float(nets[0].num_batches), float(layers[0].gamma.temperature)
+        self.lrs = [float(rates[name]) for name in SIM_PARAM_NAMES]
+        self.seed = int(seed)
+        self.X = X.detach().to(torch.float32).contiguous()
+        self.y = y.detach().to(torch.float32).contiguous()
+        self.P = (3 * in_f + 8 + 3) // 4 * 4
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.flat = torch.zeros(R, self.P, **f32)
+        self.grads = torch.zeros(R, self.P, **f32) if materialize_grads else None
+        self.step = torch.zeros(R, dtype=torch.int64, device=dev)
+        self._offsets = {}
+        off = 0
+        for name in SIM_PARAM_NAMES:
+            self._offsets[name] = off
+            off += getattr(layers[0], name).numel()
+        with torch.no_grad():
+            for r, l in enumerate(layers):
+                for name in SIM_PARAM_NAMES:
+                    p = getattr(l, name)
+                    o, k = self._offsets[name], p.numel()
+                    view = self.flat[r, o:o + k].view(p.shape)
+                    view.copy_(p.data)
+                    p.data = view
+                    if self.grads is not None:
+                        p.grad = self.grads[r, o:o + k].view(p.shape)
+
+    @staticmethod
+    def _flags_of(layers):
+        def one(l):
+            return (K.MF_FLAG_EXACT_GAMMA if l.gamma.exact else 0) | (K.MF_FLAG_EXACT_WPRIOR if l.weight_prior.exact else 0) \
+                | (K.MF_FLAG_EXACT_GPRIOR if l.gamma_prior.exact else 0)
+        flags = {one(l) for l in layers}
+        if len(flags) != 1:
+            raise K.LbbnnError("the replicas' .exact flags (gamma, weight_prior, gamma_prior) differ")
+        return flags.pop()
+
+    def steps_per_epoch(self):
+        return self.rows // self.batch
+
+    def run(self, epochs, noise=None):
+        """Train every replica for `epochs` epochs in one launch on the current stream; returns the (R, steps, 4) device tensor
+        of [loss, nll, log_prior, log_q] per step.  noise: injected draws instead of Philox (tests) -- a dict of eps_w
+        (R, steps, in), eps_b, g0_w, g0_b (R, steps) and exactly one of u (R, steps, in) or gamma (R, steps, in): constant masks,
+        no gradient through gamma."""
+        epochs = int(epochs)
+        if epochs < 1:
+            raise K.LbbnnError(f"epochs must be >= 1, got {epochs}")
+        flags = self._flags_of(self.layers)
+        R, in_f, steps = self.R, self.in_features, epochs * self.steps_per_epoch()
+        stats = torch.empty(R, steps, 4, dtype=torch.float32, device=self.flat.device)
+        d = K.MfSim()
+        d.replicas, d.in_features, d.rows, d.batch = R, in_f, self.rows, self.batch
+        d.params, d.param_stride = K.ptr(self.flat), self.P
+        d.x, d.x_stride = K.ptr(self.X), (self.rows * in_f if self.X.dim() == 3 else 0)
+        d.y, d.y_stride = K.ptr(self.y), (self.rows if self.y.dim() == 2 else 0)
+        d.lr = (C.c_float * 11)(*self.lrs)
+        d.num_batches, d.temperature, d.flags = self.num_batches, self.temperature, flags
+        d.seed = self.seed & (2 ** 64 - 1)
+        d.step = K.ptr(self.step, torch.int64)
+        d.stats, d.grads = K.ptr(stats), K.ptr(self.grads, allow_none=True)
+        keep = []
+        if noise is not None:
+            if set(noise) - set(_SIM_NOISE) - {"u", "gamma"} or not set(_SIM_NOISE) <= set(noise) \
+                    or ("u" in noise) == ("gamma" in noise):
+                raise K.LbbnnError("injected noise: eps_w, eps_b, g0_w, g0_b and exactly one of u / gamma")
+            for name, t in noise.items():
+                want = (R, steps, in_f) if name in ("eps_w", "u", "gamma") else (R, steps)
+                t = t.to(torch.float32).contiguous()
+                if tuple(t.shape) != want:
+                    raise K.LbbnnError(f"injected {name} must be {want}, got {tuple(t.shape)}")
+                keep.append(t)
+                setattr(d, name, K.ptr(t))
+        K.check(K.lib.lbbnn_mfsim_train_f32(C.byref(d), epochs, K.current_stream()))
+        return stats
+
+    def inclusion_probabilities(self):
+        """alpha = 1 / (1 + exp(-lambda)) of every replica, (R, in): what the study reports per repetition (MFsim:347-350)."""
+        o = self._offsets["lambdal"]
+        return 1.0 / (1.0 + torch.exp(-self.flat[:, o:o + self.in_features]))
 
 
 class _McLane:

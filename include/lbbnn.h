@@ -395,6 +395,47 @@ LBBNN_API int lbbnn_mf_prior_bwd_tau(const float* sums5, const float* a, const f
                                      const float* dtau_b_da, const float* dtau_b_db, float* d_scalars10, float* d_bias_a,
                                      float* d_bias_b, float* d_tau_b, float* d_bias_mu, float* d_bias_rho, lbbnn_stream s);
 
+/* ---- simulation study (LBBNN-GP-MFsim_study.py) in one launch -------------------------------------------
+ * lbbnn_mfsim_train_f32 replaces the study's repetition loop (MFsim:344-429): for each of `replicas` independent
+ * in_features -> 1 sim-study networks, `epochs` epochs of SimStudyNetwork.sample_elbo (MFsim:272-300, SAMPLES = 1: gamma
+ * rsample, w = gamma (mu + sigma eps), the Gamma precisions, log prior / log q at the unmasked ws, sigmoid + BCELoss(sum),
+ * loss = nll + (log q - log prior) / num_batches), its backward and torch.optim.SGD with one learning rate per tensor
+ * (MFsim:359-374).  One CTA per replica, parameters in registers; no allocation, no host synchronisation.
+ *   params   (replicas, param_stride), updated in place; row = weight_mu, weight_rho, lambdal (in_features each), bias_mu,
+ *            bias_rho, weight_a, weight_b, bias_a, bias_b, pa, pb; lr[] follows the same order of the 11 tensors
+ *   x, y     minibatch k of an epoch is rows [k batch, (k + 1) batch) of x (rows, in) and of the {0, 1} targets y (rows);
+ *            stride 0 = shared by every replica, rows * in_features / rows = one copy per replica
+ *   step     (replicas) int64 step counters: native noise is Philox keyed by (seed, replica, step, kind of draw), so a run
+ *            of 4 epochs equals two runs of 2 and a replica's draws do not depend on `replicas`; advanced by the launch
+ *   eps_w .. injected noise instead, all (replicas, steps, in) / (replicas, steps) with steps = epochs * rows / batch:
+ *            eps_w, eps_b, the standard-Gamma draws g0_w, g0_b and exactly one of u (relaxed / hard mask uniform) or gamma
+ *            (constant masks, no gradient through gamma); all NULL = native noise
+ *   flags    LBBNN_MF_FLAG_EXACT_GAMMA / _EXACT_WPRIOR / _EXACT_GPRIOR (the modules' .exact switches)
+ *   stats    (replicas, steps, 4): loss, nll, log_prior, log_q of every step; grads (replicas, param_stride) or NULL: the
+ *            gradients of the launch's last step */
+#define LBBNN_MFSIM_MAX_IN 32
+typedef struct lbbnn_mfsim {
+  int64_t replicas, in_features, rows, batch;
+  float* params;
+  int64_t param_stride;
+  const float* x;
+  int64_t x_stride;
+  const float* y;
+  int64_t y_stride;
+  float lr[11];
+  float num_batches, temperature;
+  int flags;
+  uint64_t seed;
+  int64_t* step;
+  const float *eps_w, *eps_b, *g0_w, *g0_b, *u, *gamma;
+  float* stats;
+  float* grads;
+} lbbnn_mfsim;
+LBBNN_API int lbbnn_mfsim_train_f32(const lbbnn_mfsim* d, int epochs, lbbnn_stream s);
+/* The standard-Gamma(a) draws of the simulation-study kernel (Marsaglia-Tsang on Philox, a < 1 boosted by U^(1/a)):
+ * out[i] is the draw `i` of stream (seed, stream_id); the kernel draws tau_w / tau_b of a step as i = 0 / 1. */
+LBBNN_API int lbbnn_philox_std_gamma(float a, int64_t n, uint64_t seed, uint64_t stream_id, float* out, lbbnn_stream s);
+
 /* ---- normalizing flows of flows2.py: PropagateFlow (flows2:14-46) over RNVP (flows2:188-219) or the
  * IAF-style MNF transform (flows2:225-241), as fused small-MLP kernels (one CTA per row of z runs the
  * whole stack; see csrc/flows.cu).  Weights are nn.Linear layout (out,in).

@@ -131,6 +131,21 @@ class MfSim(C.Structure):
         (n, C.c_void_p) for n in ("eps_w", "eps_b", "g0_w", "g0_b", "u", "gamma", "stats", "grads")]
 
 
+MNFSIM_MAX_IN, MNFSIM_MAX_T, MNFSIM_MAX_H = 32, 4, 64
+MNFSIM_DRAW_EPS_Z, MNFSIM_DRAW_EPS_Z2, MNFSIM_DRAW_EPS, MNFSIM_DRAW_EPS_R = 0, 1, 2, 3
+MNFSIM_DRAW_Z_MASK, MNFSIM_DRAW_Z_MASK2, MNFSIM_DRAW_R_MASK = 4, 8, 12
+
+
+class MnfSim(C.Structure):
+    _fields_ = [("replicas", C.c_int64), ("in_features", C.c_int64), ("rows", C.c_int64), ("batch", C.c_int64),
+                ("n_transforms", C.c_int), ("n_hidden", C.c_int), ("hidden", C.c_int * FLOW_MAX_HIDDEN),
+                ("params", C.c_void_p), ("exp_avg", C.c_void_p), ("exp_avg_sq", C.c_void_p), ("param_stride", C.c_int64),
+                ("x", C.c_void_p), ("x_stride", C.c_int64), ("y", C.c_void_p), ("y_stride", C.c_int64),
+                ("lr", C.c_float * 12), ("beta1", C.c_float), ("beta2", C.c_float), ("adam_eps", C.c_float),
+                ("num_batches", C.c_float), ("priors", Priors), ("seed", C.c_uint64), ("step", C.c_void_p)] + [
+        (n, C.c_void_p) for n in ("eps_z", "eps_z2", "z_masks", "z_masks2", "r_masks", "eps", "eps_r", "stats", "grads")]
+
+
 _P, _I64, _U64, _INT, _F, _SZ = C.c_void_p, C.c_int64, C.c_uint64, C.c_int, C.c_float, C.c_size_t
 
 # name -> (restype, argtypes); kept in one table so tests can check every header symbol is bound
@@ -250,6 +265,8 @@ SIGNATURES = {
     "lbbnn_vd_kl": (_INT, [_P, _I64, _P, _INT, _P, _F, _P]),
     "lbbnn_mfsim_train_f32": (_INT, [C.POINTER(MfSim), _INT, _P]),
     "lbbnn_philox_std_gamma": (_INT, [_F, _I64, _U64, _U64, _P, _P]),
+    "lbbnn_mnfsim_train_f32": (_INT, [C.POINTER(MnfSim), _INT, _P]),
+    "lbbnn_mnfsim_param_count": (_I64, [_I64, _INT, _INT, C.POINTER(C.c_int)]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -13,6 +13,7 @@ Reference quirks kept (SURVEY.md §0 #4): one z (the last batch row's) is broadc
 that row is pushed through the flow; the KL branch draws its own z (self.z becomes (1,in)); z_b[-1] in
 log r_b is the last ELEMENT of the flowed vector; log pi (not log 2 pi) in both Gaussians.
 """
+import ctypes as C
 import os
 
 import torch
@@ -473,3 +474,210 @@ class BayesianNetwork(nn.Module):
         updates everything else while that node runs."""
         l = self.layers[0]
         return [l.q0_mean, l.q0_log_var, *l.z_flow.parameters()]
+
+
+# the sim study's layer (MNFsim:145-251 through BayesianLinear's keyword arguments; flows_simstudy hidden sizes [50] * 5)
+SIM_LAYER_DEFAULTS = dict(mu_prior=0.1, sigma_prior=1.3, alpha_prior=0.3, bias_sigma_prior=1.3, lambda_init=(1.5, 2.5),
+                          h_sizes=(50,) * 5)
+
+
+class SimStudyNetwork(nn.Module):
+    """The MNF simulation-study model (LBBNN-GP-MF-MNFsim_study.py): one MNF layer in_features -> 1 with two RNVP
+    transforms per flow, as a logistic regression.  `layer_kwargs` override SIM_LAYER_DEFAULTS (and num_transforms).
+
+    Stated assumption: the reference script is not part of this project, and what is recorded of it is the model ("MNF
+    layer as 20 -> 1 logistic regression"), its `train` (MNFsim:272-298) and an LR-staged Adam (MNFsim:321-384).  The
+    objective below is therefore the mean-field study's (sigmoid output and BCELoss(sum), MFsim:258, 287) with the MNF
+    layer's kl in place of log q - log p, in the MNF script's train form (MNF:263-275):
+    loss = BCE(sigmoid(l1(x)), y, sum) + kl / num_batches."""
+
+    def __init__(self, in_features=20, num_batches=5.0, **layer_kwargs):
+        super().__init__()
+        kw = dict(SIM_LAYER_DEFAULTS)
+        kw.update(layer_kwargs)
+        num_transforms = kw.pop("num_transforms", 2)
+        self.l1 = BayesianLinear(in_features, 1, num_transforms, **kw)
+        self.num_batches = num_batches
+
+    def forward(self, x, sample=False, noise=None):
+        return torch.sigmoid(self.l1(x, sample, noise=noise))
+
+    def kl(self):
+        return self.l1.kl
+
+    def loss(self, x, y, noise=None):
+        """One training objective on a minibatch (sampled forward, kl computed).  Returns (loss, nll, kl)."""
+        out = torch.sigmoid(self.l1(x, True, calculate_log_probs=True, noise=noise))
+        nll = F.binary_cross_entropy(out, y.reshape(out.shape).to(out.dtype), reduction="sum")
+        kl = self.kl()
+        return nll + kl / self.num_batches, nll, kl
+
+
+# the ten layer tensors in the packed order of lbbnn_mnfsim (include/lbbnn.h), then the two flows: the 12 Adam groups
+SIM_LAYER_NAMES = ("weight_mu", "weight_rho", "lambdal", "bias_mu", "bias_rho", "q0_mean", "q0_log_var", "r0_c", "r0_b1", "r0_b2")
+SIM_GROUPS = SIM_LAYER_NAMES + ("z_flow", "r_flow")
+_SIM_NOISE = ("eps_z", "eps_z2", "z_masks", "z_masks2", "r_masks", "eps", "eps_r")
+
+
+def _flow_arch(flow):
+    """(kind, number of transforms, hidden widths) of a PropagateFlow."""
+    hidden, _, _ = flow.transforms[0].linears()
+    return flow.kind, len(flow.transforms), tuple(m.out_features for m in hidden)
+
+
+class SimStudyEnsemble:
+    """Every repetition of the MNF simulation study trained in ONE kernel launch (csrc/mnf_sim.cu): R SimStudyNetwork
+    replicas, each running the sampled forward, kl, loss = nll + kl / num_batches, its backward and torch.optim.Adam (betas
+    (0.9, 0.999), eps 1e-8, one learning rate per group) for whole epochs over minibatches of `batch_size` consecutive rows.
+
+    The replicas' parameters live in one packed (R, P) device buffer `flat` (ten layer tensors, then the z flow's and the r
+    flow's parameters); every nn.Parameter is re-pointed at a view of it (and, with materialize_grads, its .grad at the
+    last step's gradients), so state_dict() and the eager SimStudyNetwork.loss keep working on each replica.  The Adam state
+    is public: exp_avg, exp_avg_sq (laid out like `flat`) and the (R,) int64 step counts; it carries over between run()
+    calls, so a staged learning-rate schedule is a sequence of run(epochs, lrs=...) calls.
+    X is (n, in) shared by every replica or (R, n, in); y the {0, 1} targets (n,) or (R, n).  lrs: one float for every
+    group, or a dict over all 12 SIM_GROUPS.  Native noise is Philox keyed by (seed, replica, the replica's step, kind of
+    draw); see include/lbbnn.h for the streams."""
+
+    BETAS, EPS = (0.9, 0.999), 1e-8
+
+    def __init__(self, nets, X, y, batch_size=400, lrs=1e-3, seed=0, materialize_grads=True):
+        nets = list(nets)
+        if not nets:
+            raise K.LbbnnError("SimStudyEnsemble needs at least one network")
+        layers = [n.l1 for n in nets]
+
+        def signature(n):
+            l = n.l1
+            pr = l.cfg.priors
+            return (l.in_features, l.out_features, _flow_arch(l.z_flow), _flow_arch(l.r_flow),
+                    (pr.mu, pr.sigma, pr.alpha, pr.bias_mu, pr.bias_sigma), l.cfg.var_mode, float(n.num_batches))
+        sig = signature(nets[0])
+        if any(signature(n) != sig for n in nets[1:]):
+            raise K.LbbnnError("the replicas differ in shape, priors, flows (kind, transforms, hidden sizes) or num_batches")
+        in_f, out_f, zarch, rarch, _, var_mode, num_batches = sig
+        if out_f != 1 or not 1 <= in_f <= K.MNFSIM_MAX_IN:
+            raise K.LbbnnError(f"the kernel trains in_features <= {K.MNFSIM_MAX_IN} -> 1 layers, got {in_f} -> {out_f}")
+        if zarch != rarch or zarch[0] != K.FLOW_RNVP:
+            raise K.LbbnnError("the z and r flows must be RNVP flows of one architecture (IAF flows are not supported)")
+        _, T, hidden = zarch
+        if T > K.MNFSIM_MAX_T or max(hidden) > K.MNFSIM_MAX_H or len(hidden) > K.FLOW_MAX_HIDDEN:
+            raise K.LbbnnError(f"flows limited to {K.MNFSIM_MAX_T} transforms and {K.FLOW_MAX_HIDDEN} hidden layers of width <= "
+                               f"{K.MNFSIM_MAX_H}, got {T} transforms of {hidden}")
+        if var_mode != K.VAR_REFERENCE:
+            raise K.LbbnnError("the kernel implements the reference weight variance (var_mode='reference') only")
+        R = len(nets)
+        if X.dim() == 2:
+            n = X.shape[0]
+        elif X.dim() == 3 and X.shape[0] == R:
+            n = X.shape[1]
+        else:
+            raise K.LbbnnError(f"X must be (n, {in_f}) or ({R}, n, {in_f}), got {tuple(X.shape)}")
+        if X.shape[-1] != in_f:
+            raise K.LbbnnError(f"X has {X.shape[-1]} features, the networks {in_f}")
+        if tuple(y.shape) not in ((n,), (R, n)):
+            raise K.LbbnnError(f"y must be ({n},) or ({R}, {n}), got {tuple(y.shape)}")
+        B = int(batch_size)
+        if B < 1 or n % B:
+            raise K.LbbnnError(f"the {n} rows are not a whole number of minibatches of {B}")
+        self.lrs = self._rates(lrs)
+        per_net = [[getattr(l, k) for k in SIM_LAYER_NAMES] + l.z_flow._params() + l.r_flow._params() for l in layers]
+        if any(not p.is_cuda for ps in per_net for p in ps) or not X.is_cuda or not y.is_cuda:
+            raise K.LbbnnError("SimStudyEnsemble takes CUDA networks and data (no CPU fallback)")
+        dev = per_net[0][0].device
+        if any(p.device != dev for ps in per_net for p in ps) or X.device != dev or y.device != dev:
+            raise K.LbbnnError("networks and data must live on one device")
+        K.require_device()
+        self.nets, self.layers, self.R, self.in_features, self.rows, self.batch = nets, layers, R, in_f, n, B
+        self.num_batches, self.n_transforms, self.hidden = num_batches, T, hidden
+        self.priors = sig[4]
+        self.seed = int(seed)
+        self.X = X.detach().to(torch.float32).contiguous()
+        self.y = y.detach().to(torch.float32).contiguous()
+        count = sum(p.numel() for p in per_net[0])
+        hid = (C.c_int * len(hidden))(*hidden)
+        assert count == K.lib.lbbnn_mnfsim_param_count(in_f, T, len(hidden), hid)
+        self.P = (count + 3) // 4 * 4
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.flat = torch.zeros(R, self.P, **f32)
+        self.exp_avg = torch.zeros(R, self.P, **f32)
+        self.exp_avg_sq = torch.zeros(R, self.P, **f32)
+        self.grads = torch.zeros(R, self.P, **f32) if materialize_grads else None
+        self.step = torch.zeros(R, dtype=torch.int64, device=dev)
+        self._lam = sum(getattr(layers[0], k).numel() for k in SIM_LAYER_NAMES[:2])
+        with torch.no_grad():
+            for r, ps in enumerate(per_net):
+                o = 0
+                for p in ps:
+                    k = p.numel()
+                    view = self.flat[r, o:o + k].view(p.shape)
+                    view.copy_(p.data)
+                    p.data = view
+                    if self.grads is not None:
+                        p.grad = self.grads[r, o:o + k].view(p.shape)
+                    o += k
+
+    @staticmethod
+    def _rates(lrs):
+        if isinstance(lrs, dict):
+            if set(lrs) != set(SIM_GROUPS):
+                raise K.LbbnnError(f"lrs must name exactly the groups {SIM_GROUPS}; unknown {sorted(set(lrs) - set(SIM_GROUPS))}, "
+                                   f"missing {sorted(set(SIM_GROUPS) - set(lrs))}")
+            return [float(lrs[g]) for g in SIM_GROUPS]
+        if isinstance(lrs, (int, float)) and not isinstance(lrs, bool):
+            return [float(lrs)] * len(SIM_GROUPS)
+        raise K.LbbnnError(f"lrs must be a float or a dict over {SIM_GROUPS}, got {type(lrs).__name__}")
+
+    def steps_per_epoch(self):
+        return self.rows // self.batch
+
+    def run(self, epochs, lrs=None, noise=None):
+        """Train every replica for `epochs` epochs in one launch on the current stream; returns the (R, steps, 3) device tensor
+        of [loss, nll, kl] per step.  lrs: new learning rates from this run on (kept for later runs).  noise: injected
+        draws instead of Philox (tests), a dict of eps_z, eps_z2 (R, steps, in), z_masks, z_masks2, r_masks
+        (R, steps, T, in), eps (R, steps, batch), eps_r (R, steps)."""
+        if isinstance(epochs, bool) or int(epochs) != epochs or epochs < 1:
+            raise K.LbbnnError(f"epochs must be an integer >= 1, got {epochs}")
+        epochs = int(epochs)
+        rates = self.lrs if lrs is None else self._rates(lrs)
+        R, D, T, steps = self.R, self.in_features, self.n_transforms, epochs * self.steps_per_epoch()
+        keep = {}
+        if noise is not None:
+            if set(noise) != set(_SIM_NOISE):
+                raise K.LbbnnError(f"injected noise takes exactly {_SIM_NOISE}, got {sorted(noise)}")
+            want = {"eps_z": (R, steps, D), "eps_z2": (R, steps, D), "z_masks": (R, steps, T, D), "z_masks2": (R, steps, T, D),
+                    "r_masks": (R, steps, T, D), "eps": (R, steps, self.batch), "eps_r": (R, steps)}
+            for name, t in noise.items():
+                if not torch.is_tensor(t) or tuple(t.shape) != want[name]:
+                    raise K.LbbnnError(f"injected {name} must be a tensor of shape {want[name]}, got "
+                                       f"{tuple(t.shape) if torch.is_tensor(t) else type(t).__name__}")
+            for name, t in noise.items():
+                if not t.is_cuda or t.device != self.flat.device:
+                    raise K.LbbnnError(f"injected {name} must live on {self.flat.device}")
+                keep[name] = t.detach().to(torch.float32).contiguous()
+        self.lrs = rates
+        stats = torch.empty(R, steps, 3, dtype=torch.float32, device=self.flat.device)
+        d = K.MnfSim()
+        d.replicas, d.in_features, d.rows, d.batch = R, D, self.rows, self.batch
+        d.n_transforms, d.n_hidden = T, len(self.hidden)
+        for i, h in enumerate(self.hidden):
+            d.hidden[i] = h
+        d.params, d.exp_avg, d.exp_avg_sq, d.param_stride = K.ptr(self.flat), K.ptr(self.exp_avg), K.ptr(self.exp_avg_sq), self.P
+        d.x, d.x_stride = K.ptr(self.X), (self.rows * D if self.X.dim() == 3 else 0)
+        d.y, d.y_stride = K.ptr(self.y), (self.rows if self.y.dim() == 2 else 0)
+        d.lr = (C.c_float * 12)(*rates)
+        d.beta1, d.beta2, d.adam_eps = self.BETAS[0], self.BETAS[1], self.EPS
+        d.num_batches = self.num_batches
+        d.priors = K.Priors(*self.priors)
+        d.seed = self.seed & (2 ** 64 - 1)
+        d.step = K.ptr(self.step, torch.int64)
+        d.stats, d.grads = K.ptr(stats), K.ptr(self.grads, allow_none=True)
+        for name, t in keep.items():
+            setattr(d, name, K.ptr(t))
+        K.check(K.lib.lbbnn_mnfsim_train_f32(C.byref(d), epochs, K.current_stream()))
+        return stats
+
+    def inclusion_probabilities(self):
+        """alpha = 1 / (1 + exp(-lambdal)) of every replica, (R, in)."""
+        o = self._lam
+        return 1.0 / (1.0 + torch.exp(-self.flat[:, o:o + self.in_features]))

@@ -474,6 +474,65 @@ LBBNN_API int lbbnn_flow_bwd(const lbbnn_flow* flow, const lbbnn_flow_grads* gra
                              const lbbnn_noise* mask_u, const float* dz_out, const float* dlogdet, const float* save,
                              float* dz_in, lbbnn_stream s);
 
+/* ---- MNF simulation study (LBBNN-GP-MF-MNFsim_study.py) in one launch ------------------------------------
+ * lbbnn_mnfsim_train_f32 trains `replicas` independent in_features -> 1 MNF logistic regressions
+ * (lbbnn.mnf.SimStudyNetwork: one MNF layer with RNVP z and r flows, sigmoid + BCELoss(sum),
+ * loss = nll + kl / num_batches) for `epochs` epochs with torch.optim.Adam, one learning rate per group.
+ * One CTA per replica; no allocation, no host synchronisation.
+ *   params   (replicas, param_stride), updated in place; a row holds weight_mu, weight_rho, lambdal, bias_mu, bias_rho,
+ *            q0_mean, q0_log_var, r0_c, r0_b1, r0_b2 (in_features each, the biases 1), then the z flow's and the r flow's
+ *            parameters in PropagateFlow._params() order (per transform: network.{0,2,..} weight, bias, t weight, bias,
+ *            s weight, bias; nn.Linear layout)
+ *   exp_avg, exp_avg_sq   Adam moments laid out like params, updated in place; lr[] = the ten layer tensors in the order
+ *            above, then the z flow, then the r flow; beta1, beta2, adam_eps as torch.optim.Adam (no weight decay)
+ *   step     (replicas) int64: Adam's step count (bias correction) and the native-noise step key; advanced by the launch
+ *   x, y     minibatch k of an epoch is rows [k batch, (k + 1) batch) of x (rows, in) and of the {0, 1} targets y (rows);
+ *            stride 0 = shared by every replica, rows * in_features / rows = one copy per replica
+ *   native noise (all injected pointers NULL): Philox (seed, stream) with stream = replica << 40 | step << 4 | kind and
+ *            step = step[replica] before the launch + the step within it; element e of a draw is element e of
+ *            lbbnn_philox_normal / lbbnn_philox_uniform of that stream.  Kinds (LBBNN_MNFSIM_DRAW_*):
+ *              EPS_Z  normal, in_features: the activation row's z0 = q0_mean + sqrt(exp(q0_log_var)) eps_z
+ *              EPS_Z2 normal, in_features: the KL row's z0
+ *              EPS    normal, batch: the LRT output noise of the minibatch rows
+ *              EPS_R  normal, element 0: the auxiliary r(z|W) noise
+ *              Z_MASK + t, Z_MASK2 + t, R_MASK + t   uniform, in_features: transform t's mask [u < 0.5] of the activation row's
+ *              z flow, of the KL row's z flow and of the r flow
+ *   injected noise instead (tests): eps_z, eps_z2 (replicas, steps, in); z_masks, z_masks2, r_masks (replicas, steps, T, in)
+ *            of {0, 1}; eps (replicas, steps, batch); eps_r (replicas, steps); steps = epochs * rows / batch
+ *   stats    (replicas, steps, 3): loss, nll, kl of every step; grads (replicas, param_stride) or NULL: the gradients of the
+ *            launch's last step
+ * Limits: in_features <= LBBNN_MNFSIM_MAX_IN, out_features = 1, RNVP flows only, n_transforms <= LBBNN_MNFSIM_MAX_T,
+ * hidden widths <= LBBNN_MNFSIM_MAX_H, n_hidden <= LBBNN_FLOW_MAX_HIDDEN. */
+#define LBBNN_MNFSIM_MAX_IN 32
+#define LBBNN_MNFSIM_MAX_T 4
+#define LBBNN_MNFSIM_MAX_H 64
+enum {
+  LBBNN_MNFSIM_DRAW_EPS_Z = 0, LBBNN_MNFSIM_DRAW_EPS_Z2 = 1, LBBNN_MNFSIM_DRAW_EPS = 2, LBBNN_MNFSIM_DRAW_EPS_R = 3,
+  LBBNN_MNFSIM_DRAW_Z_MASK = 4, LBBNN_MNFSIM_DRAW_Z_MASK2 = 8, LBBNN_MNFSIM_DRAW_R_MASK = 12
+};
+typedef struct lbbnn_mnfsim {
+  int64_t replicas, in_features, rows, batch;
+  int n_transforms, n_hidden;
+  int hidden[LBBNN_FLOW_MAX_HIDDEN];
+  float *params, *exp_avg, *exp_avg_sq;
+  int64_t param_stride;
+  const float* x;
+  int64_t x_stride;
+  const float* y;
+  int64_t y_stride;
+  float lr[12];
+  float beta1, beta2, adam_eps, num_batches;
+  lbbnn_priors priors;
+  uint64_t seed;
+  int64_t* step;
+  const float *eps_z, *eps_z2, *z_masks, *z_masks2, *r_masks, *eps, *eps_r;
+  float* stats;
+  float* grads;
+} lbbnn_mnfsim;
+LBBNN_API int lbbnn_mnfsim_train_f32(const lbbnn_mnfsim* d, int epochs, lbbnn_stream s);
+/* floats of one packed parameter row of lbbnn_mnfsim (before padding) */
+LBBNN_API int64_t lbbnn_mnfsim_param_count(int64_t in_features, int n_transforms, int n_hidden, const int* hidden);
+
 /* ---- MNF auxiliary KL terms (MNF:208-235 minus the flows and the weight KL; csrc/mnf_aux.cu) -----------------------
  * out3 = [log_q0 - log_rb, log_q0, log_rb] with
  *   log_q0 = sum_i -0.5 log(pi) - 0.5 q0_log_var_i - 0.5 (z0_i - q0_mean_i)^2 / exp(q0_log_var_i)          (MNF:212-214)

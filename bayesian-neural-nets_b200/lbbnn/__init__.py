@@ -5,10 +5,10 @@ from . import _capi
 from ._capi import LbbnnError, philox_normal, philox_uniform
 from .lrt import BayesianLinear, BayesianNetwork, LayerConfig, lrt_linear, manual_seed, predict_ensemble
 from . import flows, mf, mnf
-from .engine import GraphedTrainer, LRTTrainer, LRTTensorCoreTrainer, MultiTensorAdam
+from .engine import GraphedTrainer, LRTReplicaTrainer, LRTTrainer, LRTTensorCoreTrainer, MultiTensorAdam
 from . import vd
 from . import predict
 from .predict import EnsemblePredictor, mf_outofsample
 
-__all__ = ["BayesianLinear", "BayesianNetwork", "GraphedTrainer", "LayerConfig", "LRTTrainer", "LRTTensorCoreTrainer", "LbbnnError", "MultiTensorAdam", "lrt_linear",
+__all__ = ["BayesianLinear", "BayesianNetwork", "GraphedTrainer", "LayerConfig", "LRTReplicaTrainer", "LRTTrainer", "LRTTensorCoreTrainer", "LbbnnError", "MultiTensorAdam", "lrt_linear",
            "manual_seed", "predict_ensemble", "predict", "EnsemblePredictor", "mf_outofsample", "mf", "mnf", "flows", "vd", "philox_normal", "philox_uniform"]

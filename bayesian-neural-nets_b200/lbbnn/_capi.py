@@ -120,6 +120,14 @@ class Step(C.Structure):
                 ("kl_scale", C.c_float), ("stats", C.c_void_p), ("dp", C.POINTER(StepDp))]
 
 
+STEP_MAX_REPLICAS = 64
+
+
+class StepReplicas(C.Structure):
+    _fields_ = [("replicas", C.c_int), ("param_stride", C.c_int64), ("x_stride", C.c_int64), ("y_stride", C.c_int64),
+                ("seeds", C.c_void_p)]
+
+
 MFSIM_MAX_IN = 32
 
 
@@ -245,6 +253,9 @@ SIGNATURES = {
     "lbbnn_lrt_step_f32": (_INT, [C.POINTER(Step), _INT, _P, _SZ, _P]),
     "lbbnn_lrt_step_profile": (_INT, [_P]),
     "lbbnn_lrt_step_describe": (_INT, [C.POINTER(Step), C.c_char_p, _SZ]),
+    "lbbnn_lrt_step_replicas_workspace_bytes": (_SZ, [C.POINTER(Step), C.POINTER(StepReplicas)]),
+    "lbbnn_lrt_step_replicas_f32": (_INT, [C.POINTER(Step), C.POINTER(StepReplicas), _P, _SZ, _P]),
+    "lbbnn_lrt_step_replicas_describe": (_INT, [C.POINTER(Step), C.POINTER(StepReplicas), C.c_char_p, _SZ]),
     "lbbnn_logsoftmax_nll_f32": (_INT, [_P, _P, _I64, _I64, _P, _P, _P, _F, _P, _P, _SZ, _P]),
     "lbbnn_adam_f32": (_INT, [_P, _P, _P, _P, _I64, _F, _F, _F, _F, _P, _P, _P]),
     "lbbnn_adam_multi_f32": (_INT, [_P, _INT, _I64, _F, _F, _F, _F, _P, _P, _P]),

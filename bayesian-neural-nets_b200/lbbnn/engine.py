@@ -53,7 +53,7 @@ def check_replicas(process_group, params, what):
 class LRTTrainer:
     def __init__(self, net, batch_size, num_batches, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, seed=None,
                  use_graph=True, inject_noise=False, process_group=None, fused=None, materialize_grads=True):
-        """fused: run the step as the single persistent kernel of csrc/lrt_step.cu (None = whenever it applies:
+        """fused: run the step as the single persistent kernel of csrc/lrt_step.cuh (None = whenever it applies:
         batch <= 128, <= 8 layers); False = one launch sequence per layer (csrc/lrt_f32.cu).
         materialize_grads: also write the parameter gradients to `.grad` (the fused kernel otherwise consumes
         them in registers inside the Adam update)."""
@@ -128,7 +128,7 @@ class LRTTrainer:
         if use_graph:
             self._capture()
 
-    # ---- fused single-kernel step (csrc/lrt_step.cu) ------------------------------------------------
+    # ---- fused single-kernel step (csrc/lrt_step.cuh) -----------------------------------------------
     def _try_dp_arena(self, n_flat, sizes):
         """LBBNN_DP_ALLREDUCE = auto | sharded: one symmetric-memory arena [parameters | step workspace | signal pad | KL
         exchange] bound to an NVSwitch multicast object, for the in-launch sharded update (lbbnn_step_dp).  Leaves
@@ -506,6 +506,171 @@ class LRTTrainer:
     @property
     def d2h_bytes_per_step(self):
         return self.stats_host.numel() * 4
+
+
+class LRTReplicaTrainer:
+    """R LRT networks of one shape trained side by side: every step of all of them is ONE launch of the persistent step
+    kernel (csrc/lrt_step.cuh, lbbnn_lrt_step_replicas_f32), whose phases run their work items over all replicas -- the
+    reference driver's seed loop (LBBNN-GP-MF-LRT.py:354-372, one network and one optim.Adam per seed) without paying the
+    step's grid barriers and phase latencies once per seed.
+
+    nets: LRT BayesianNetworks with the same sizes, per-layer priors and var_mode, on one CUDA device.  Replica r's parameters,
+    gradients and Adam moments are row r of (R, P) buffers (`flat`, `gflat`, `exp_avg`, `exp_avg_sq`), each row with
+    LRTTrainer's flat layout; every nn.Parameter (and its .grad) is re-pointed at a view of its row, so state_dict(), eager
+    forward and EnsemblePredictor(net) keep working on each net.  seeds: replica r draws the noise LRTTrainer(net, seed=seeds[r])
+    draws (default lbbnn.lrt.current_seed() + r).  shared_batch: one (B, ...) minibatch for all replicas instead of (R, B, ...).
+    Each replica's parameters, moments and gradients equal LRTTrainer's under the same schedule bit for bit."""
+
+    def __init__(self, nets, batch_size, num_batches, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, seeds=None,
+                 shared_batch=False, use_graph=True, inject_noise=False, materialize_grads=True):
+        nets = list(nets)
+        R = len(nets)
+        if not 1 <= R <= K.STEP_MAX_REPLICAS:
+            raise K.LbbnnError(f"LRTReplicaTrainer: 1..{K.STEP_MAX_REPLICAS} networks, got {R}")
+        for r, net in enumerate(nets):
+            if not isinstance(net, _lrt.BayesianNetwork) or not all(isinstance(l, _lrt.BayesianLinear) for l in net.layers):
+                raise K.LbbnnError(f"LRTReplicaTrainer: nets[{r}] is not an LRT BayesianNetwork")
+        sizes = tuple(nets[0].sizes)
+        cfg = lambda net: [(tuple(getattr(l.cfg.priors, f) for f, _ in K.Priors._fields_), l.cfg.var_mode)  # noqa: E731
+                           for l in net.layers]
+        for r, net in enumerate(nets):
+            if tuple(net.sizes) != sizes:
+                raise K.LbbnnError(f"LRTReplicaTrainer: nets[{r}] has sizes {tuple(net.sizes)}, nets[0] {sizes}")
+            if cfg(net) != cfg(nets[0]):
+                raise K.LbbnnError(f"LRTReplicaTrainer: nets[{r}] differs from nets[0] in a layer's priors or var_mode")
+        self.B = int(batch_size)
+        if not 1 <= self.B <= 128 or len(sizes) - 1 > K.STEP_MAX_LAYERS:
+            raise K.LbbnnError("LRTReplicaTrainer: the step kernel needs batch 1..128 and <= 8 layers "
+                               f"(got batch {self.B}, {len(sizes) - 1} layers)")
+        seeds = [_lrt.current_seed() + r for r in range(R)] if seeds is None else [int(v) for v in seeds]
+        if len(seeds) != R or any(not 0 <= v < 2 ** 64 for v in seeds):
+            raise K.LbbnnError(f"LRTReplicaTrainer: need {R} seeds in [0, 2**64), got {seeds}")
+        devs = {p.device for net in nets for p in net.parameters()}
+        if len(devs) != 1 or next(iter(devs)).type != "cuda":
+            raise K.LbbnnError(f"LRTReplicaTrainer: every net must live on one CUDA device (got {sorted(map(str, devs))})")
+        K.require_device()
+        self.nets, self.R, self.seeds = nets, R, seeds
+        self.num_batches = int(num_batches)
+        self.lr, self.betas, self.eps = float(lr), betas, float(eps)
+        self.shared_batch, self.materialize_grads = bool(shared_batch), bool(materialize_grads)
+        self.device = dev = next(iter(devs))
+        layers0 = nets[0].layers
+        L = len(layers0)
+
+        # ---- (R, P) parameter / gradient / Adam-state storage: row r = LRTTrainer's flat layout of nets[r] ----
+        offs, total = [], 0
+        for i, l in enumerate(layers0):
+            for name in _PARAM_NAMES:
+                n = getattr(l, name).numel()
+                offs.append((i, name, total, n))
+                total += _pad4(n)
+        self.n_flat = total
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.flat = torch.zeros(R, total, **f32)
+        self.gflat = torch.zeros(R, total, **f32)
+        self.exp_avg = torch.zeros(R, total, **f32)
+        self.exp_avg_sq = torch.zeros(R, total, **f32)
+        self.step_dev = torch.zeros(1, dtype=torch.int64, device=dev)
+        with torch.no_grad():
+            for r, net in enumerate(nets):
+                for i, name, off, n in offs:
+                    p = getattr(net.layers[i], name)
+                    view = self.flat[r, off:off + n].view(p.shape)
+                    view.copy_(p.data)
+                    p.data = view
+                    p.grad = self.gflat[r, off:off + n].view(p.shape)
+        self._offsets = {(i, name): off for i, name, off, n in offs}
+
+        # ---- minibatches, noise, stats ----
+        lead = () if self.shared_batch else (R,)
+        self.x = torch.zeros(*lead, self.B, sizes[0], **f32)
+        self.y = torch.zeros(*lead, self.B, dtype=torch.int64, device=dev)
+        self.eps_in = [torch.zeros(R, self.B, o, **f32) for o in sizes[1:]] if inject_noise else None
+        self.stats = torch.zeros(R, 1 + L, **f32)
+        # uint64 seeds as their int64 bit patterns
+        self.seeds_dev = torch.tensor([v - 2 ** 64 if v >= 2 ** 63 else v for v in seeds], dtype=torch.int64, device=dev)
+        st = K.Step()
+        st.n_layers, st.batch = L, self.B
+        for i, l in enumerate(layers0):
+            sl = st.layer[i]
+            sl.in_features, sl.out_features = l.in_features, l.out_features
+            sl.off_weight_mu, sl.off_weight_rho, sl.off_lambdal, sl.off_bias_mu, sl.off_bias_rho = (
+                self._offsets[(i, n)] for n in _PARAM_NAMES)
+            sl.eps = K.ptr(self.eps_in[i]) if inject_noise else None
+            sl.priors, sl.var_mode = l.cfg.priors, l.cfg.var_mode
+        st.flat, st.exp_avg, st.exp_avg_sq = K.ptr(self.flat), K.ptr(self.exp_avg), K.ptr(self.exp_avg_sq)
+        st.grad = K.ptr(self.gflat) if self.materialize_grads else None
+        st.x, st.y, st.step_dev = K.ptr(self.x), K.ptr(self.y, torch.int64), K.ptr(self.step_dev, torch.int64)
+        st.lr, st.beta1, st.beta2, st.eps = self.lr, self.betas[0], self.betas[1], self.eps
+        st.kl_scale = 1.0 / self.num_batches
+        st.stats = K.ptr(self.stats)
+        rp = K.StepReplicas()
+        rp.replicas, rp.param_stride = R, total
+        rp.x_stride = 0 if self.shared_batch else self.B * sizes[0]
+        rp.y_stride = 0 if self.shared_batch else self.B
+        rp.seeds = K.ptr(self.seeds_dev, torch.int64)
+        self._step_desc, self._replicas = st, rp
+        nbytes = int(K.lib.lbbnn_lrt_step_replicas_workspace_bytes(st, rp))
+        if nbytes == 0:
+            raise K.LbbnnError("replica step: " + K.lib.lbbnn_last_error().decode())
+        self.ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)   # zero-filled once (the barrier ticket lives in it)
+        buf = C_create_string_buffer(4096)
+        K.check(K.lib.lbbnn_lrt_step_replicas_describe(st, rp, buf, 4096))
+        self.schedule = buf.value.decode()
+        self.x_host = torch.zeros(self.x.shape, dtype=torch.float32).pin_memory()
+        self.y_host = torch.zeros(self.y.shape, dtype=torch.int64).pin_memory()
+        self.stats_host = torch.zeros(R, 1 + L, dtype=torch.float32).pin_memory()
+        self.kernels_per_step = 1
+        self.graph = None
+        if use_graph:
+            self._capture()
+
+    def _enqueue(self):
+        K.check(K.lib.lbbnn_lrt_step_replicas_f32(self._step_desc, self._replicas, self.ws.data_ptr(), self.ws.numel(),
+                                                  K.current_stream()))
+
+    def _capture(self):
+        # side-stream warm-up, undone (it must not count as training), then capture -- as LRTTrainer._capture
+        tensors = (self.flat, self.exp_avg, self.exp_avg_sq, self.step_dev)
+        state = [t.clone() for t in tensors]
+        s = torch.cuda.Stream(device=self.device)
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            self._enqueue()
+        torch.cuda.current_stream().wait_stream(s)
+        torch.cuda.synchronize()
+        for t, saved in zip(tensors, state):
+            t.copy_(saved)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self._enqueue()
+
+    def step_device(self):
+        """One training step of every replica on the minibatches already in self.x / self.y (device resident)."""
+        if self.graph is not None:
+            self.graph.replay()
+        else:
+            self._enqueue()
+
+    def step(self, x_host, y_host, read_loss=True):
+        """One training step of every replica from HOST tensors: x (R, B, ...) and y (R, B), or (B, ...) and (B,) with
+        shared_batch.  Returns {"nll", "kl", "loss"} as length-R lists (None when read_loss is False)."""
+        lead = () if self.shared_batch else (self.R,)
+        if tuple(y_host.shape) != lead + (self.B,) or x_host.numel() != self.x.numel():
+            raise K.LbbnnError(f"LRTReplicaTrainer.step: expected x of {tuple(self.x.shape)} elements' shape and y of shape "
+                               f"{lead + (self.B,)}, got {tuple(x_host.shape)} and {tuple(y_host.shape)}")
+        self.x_host.copy_(x_host.reshape(self.x_host.shape))
+        self.y_host.copy_(y_host)
+        self.x.copy_(self.x_host, non_blocking=True)
+        self.y.copy_(self.y_host, non_blocking=True)
+        self.step_device()
+        if not read_loss:
+            return None
+        self.stats_host.copy_(self.stats, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        nll = self.stats_host[:, 0].tolist()
+        kl = self.stats_host[:, 1:].sum(dim=1).tolist()
+        return {"nll": nll, "kl": kl, "loss": [a + b / self.num_batches for a, b in zip(nll, kl)]}
 
 
 class LRTTensorCoreTrainer:

@@ -647,6 +647,39 @@ LBBNN_API int lbbnn_lrt_step_profile(long long* dev_stamps);
 /* human-readable schedule (tile sizes / work items per phase) chosen for this step */
 LBBNN_API int lbbnn_lrt_step_describe(const lbbnn_step* step, char* buf, size_t buf_bytes);
 
+/* ---- R networks of one shape trained side by side in ONE launch of the same persistent kernel ----------------------
+ * The reference's driver trains one network per seed (LRT:354-372); here every phase's work items run over all replicas
+ * (replica-major), so the step's grid barriers and phase latencies are paid once for the R networks.  The lbbnn_step
+ * supplies what the replicas share: the shapes, each layer's float offsets WITHIN one replica, priors and var_mode, lr, the
+ * betas, eps, kl_scale, and the base pointers (replica 0's).  Under these entry points:
+ *   - replica r's parameters, Adam state and (optional) gradients sit r * param_stride floats after the base pointers;
+ *   - its minibatch is x + r * x_stride, y + r * y_stride (elements; 0 = one minibatch shared by all replicas);
+ *   - stats holds R rows of 1 + n_layers floats, [nll, kl_1 .. kl_L] of replica r in row r;
+ *   - step_dev is ONE counter: the replicas step in lockstep, and it is incremented once per launch;
+ *   - layer i's injected eps, when not NULL, points at an (R, batch, out_i) tensor; otherwise replica r draws
+ *     Philox(seeds[r], stream = i + step * n_layers) at the element index within the replica -- exactly the noise a single
+ *     network with seed seeds[r] draws through lbbnn_lrt_step_f32;  `seed` is ignored;
+ *   - dp must be NULL; the launch is always the full step (phases 3).
+ * Each replica's parameters, moments and gradients equal those of lbbnn_lrt_step_f32 with seed seeds[r] under the same
+ * schedule bit for bit; its nll and KL sums may be taken in another order.  The workspace must be zero-filled once before its
+ * first use and is otherwise opaque; lbbnn_lrt_step_replicas_workspace_bytes returns 0 (and sets lbbnn_last_error) when an
+ * argument is out of range. */
+#define LBBNN_STEP_MAX_REPLICAS 64
+typedef struct lbbnn_step_replicas {
+  int replicas;                 /* R >= 1, <= LBBNN_STEP_MAX_REPLICAS */
+  int64_t param_stride;         /* floats between replicas in flat / exp_avg / exp_avg_sq / grad; multiple of 4, covers
+                                   every layer's tensors */
+  int64_t x_stride, y_stride;   /* elements between replicas' minibatches; 0 = one minibatch shared by all */
+  const uint64_t* seeds;        /* device, R: replica r draws Philox(seeds[r], ...) */
+} lbbnn_step_replicas;
+LBBNN_API size_t lbbnn_lrt_step_replicas_workspace_bytes(const lbbnn_step* step, const lbbnn_step_replicas* replicas);
+LBBNN_API int lbbnn_lrt_step_replicas_f32(const lbbnn_step* step, const lbbnn_step_replicas* replicas, void* workspace,
+                                          size_t workspace_bytes, lbbnn_stream s);
+/* the schedule of the replica launch: lbbnn_lrt_step_describe's format with per-replica item counts, followed by
+ * " replicas=R" when R > 1 (R = 1 prints exactly the single-network string) */
+LBBNN_API int lbbnn_lrt_step_replicas_describe(const lbbnn_step* step, const lbbnn_step_replicas* replicas, char* buf,
+                                               size_t buf_bytes);
+
 /* ---- loss head: F.log_softmax(dim=1) + F.nll_loss(reduction='sum') (LRT:210,223) ------------
  * logp (batch,classes) and dlogits (batch,classes) = grad_scale*(softmax - onehot) may be NULL.
  * step_inc (device int64 or NULL) is incremented by one: the trainer's step counter, bumped between
